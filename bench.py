@@ -1,8 +1,8 @@
 #!/usr/bin/env python
 """bench.py -- env-steps/s INCLUDING Q-updates (BASELINE.json metric) on N B200s of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-    (N > 1: launched by the driver as  python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...)
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
+    (N > 1: one process per GPU, as  python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...)
 
 Workload (BASELINE.json configs[4], one GPU's shard; named in config.workload): independent agent
 populations (seed x platform-speed x learning-rate sweep), x axis, curriculum step 0, ~1M envs per GPU,
@@ -15,6 +15,8 @@ ranks.  `e2e` = the same metric through the C-ABI host-buffer entry point dqlb20
 env-state + tables + trainer state copied in, E2E_CHUNK global steps, everything copied back, every call).
 `cpu_baseline` = the reference's single-env Python loop (oracle port) on one host core, bounded sample.
 `--impl reference` = that loop on every host core.
+`--dump-outputs DIR` = after the timed steps, what they left to the caller as DIR/<name>.npy (see dump_outputs); the inputs
+are fixed by the arguments, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -39,6 +41,9 @@ THREADS_PER_BLOCK = 128
 E2E_CHUNK = 64                     # global steps per host-buffer call (about one episode, the reference's save interval)
 E2E_TABLE_LEVELS = 2               # curriculum step 0 with promotions off: levels 0 (live) and 1 (next) of the tables travel, checked by the library
 ALGORITHMIC_BYTES_PER_ENV_STEP = 96   # SURVEY.md 8(d): 48 B env state read + 48 B written, one step per launch
+RAMP_LAUNCHES = 356                # untimed clock ramp, 32 global steps each: 0.3 s on a B200 at 1,965 MHz, 1,000 W power limit
+DUMP_ENVS = 65536                  # --dump-outputs: env states of this many envs, a fixed seeded sample
+DUMP_MAX_BYTES = 64 << 20
 
 
 SHARED_SYNC_EVERY = 16             # global steps between two shared-table all-reduces (N > 1 only)
@@ -61,6 +66,35 @@ def workload_config(n_gpus: int) -> dict:
         "rng": "Philox4x32-10, key = seed (5 seeds per sweep point), counter word 3 = global population id", "platform_speeds": [0.4, 0.8, 1.2, 1.6],
         "alpha_variants": [[0.02949, 0.51], [0.05, 0.6]],
     }
+
+
+def dump_outputs(eng, out: pathlib.Path, np):
+    """What the timed training steps leave to their caller, read back after the last one and written as out/<name>.npy:
+    the Q-table pair and visit counts of every population (all curriculum levels), the trainer state of every population, and the
+    env state of DUMP_ENVS envs drawn with a fixed seed (the whole env state is 54 MB of packed words; the sample keeps the dump
+    small).  Everything is float32 (what the kernel holds as float32) or float64 (exact for the integers and the float64 sums)."""
+    t = eng.tables.cpu().numpy().view(np.uint32)                    # [population][q_a, q_b, count][MAX_CELLS]
+    arrays = {"q_a": t[:, 0].view(np.float32), "q_b": t[:, 1].view(np.float32), "count": t[:, 2].astype(np.float64)}
+    ps = eng.population_state()
+    for f in ps.dtype.names:
+        arrays["population_" + f] = ps[f].astype(np.float64)
+    # env layout [population][tile of 32 envs][vector A, B, C][env in tile][4 words]; fields as in env_unpack (csrc/env_state.cuh)
+    w = eng.env_state.view(eng.P, eng.tiles_per_population, 3, 32, 4).cpu().numpy().view(np.uint32)
+    pick = np.sort(np.random.default_rng(0).choice(eng.n_total, min(DUMP_ENVS, eng.n_total), replace=False))
+    pop, env = pick // eng.n_p, pick % eng.n_p
+    e = w[pop, env // 32, :, env % 32]                              # [n][A, B, C][4 words]
+    arrays["env_index"] = pick.astype(np.float64)                   # population * envs_per_population + env
+    arrays["env_body"] = e[:, 0, :3].view(np.float32)               # x_d, v_d, theta
+    arrays["env_prev_rel"] = e[:, 1, 2:].view(np.float32)           # previous rel_p, rel_v (reward shaping)
+    # platform phase, set-point index, packed word (state id, step count, curriculum check, flags, position bin), episode
+    arrays["env_words"] = np.stack([e[:, 0, 3], e[:, 1, 0], e[:, 2, 0], e[:, 2, 1]], axis=1).astype(np.float64)
+    arrays["env_cum_reward"] = np.ascontiguousarray(e[:, 2, 2:]).view(np.float64)[:, 0]
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES}-byte limit")
+    out.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(out / f"{name}.npy", np.ascontiguousarray(a))
 
 
 # ----------------------------------------------------------------------------------------------------
@@ -263,9 +297,9 @@ def run_ours(args, rank: int, local_rank: int, world: int):
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
     stream = torch.cuda.current_stream(dev)
 
-    # clock ramp (untimed, not counted as warm-up steps): ~0.3 s of the same kernel
-    t_end = time.perf_counter() + (0.0 if os.environ.get("DQL_BENCH_NO_RAMP") else 0.3)
-    while time.perf_counter() < t_end:
+    # clock ramp (untimed, not counted as warm-up steps): a fixed number of launches of the same kernel, so that the timed steps
+    # start from the same state in every run with the same arguments
+    for _ in range(0 if os.environ.get("DQL_BENCH_NO_RAMP") else RAMP_LAUNCHES):
         eng.train(32)
         torch.cuda.synchronize(dev)
     sampler = ClockSampler(local_rank)
@@ -285,6 +319,8 @@ def run_ours(args, rank: int, local_rank: int, world: int):
     barrier()
     ms = sum(a.elapsed_time(b) for a, b in ev)
     eng.check_errors()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(eng, pathlib.Path(args.dump_outputs), np)
 
     # ---- e2e: host buffers through dqlb200_train_host ----------------------------------------------
     env_h = torch.empty_like(eng.env_state, device="cpu").pin_memory()
@@ -722,7 +758,13 @@ def main():
     ap.add_argument("--impl", choices=["ours", "reference"], default="ours")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-extra", action="store_true", help="skip the other-config measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (rank 0's populations)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -738,6 +780,7 @@ def main():
                "--gpus", str(args.gpus), "--steps", str(args.steps), "--warmup", str(args.warmup)]
         cmd += ["--no-cpu"] if args.no_cpu else []
         cmd += ["--no-extra"] if args.no_extra else []
+        cmd += ["--dump-outputs", os.path.abspath(args.dump_outputs)] if args.dump_outputs else []
         sys.exit(subprocess.call(cmd))
     run_ours(args, rank, local_rank, world)
 
