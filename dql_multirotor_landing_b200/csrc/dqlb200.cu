@@ -259,6 +259,18 @@ int dqlb200_bind(dqlb200_handle* h, void* env_state, void* tables, void* pop_sta
   if (!h || !env_state || !tables || !pop_state) return fail(DQLB200_ERR_ARG, "null argument");
   if (((uintptr_t)env_state & 15u) || ((uintptr_t)tables & 3u) || ((uintptr_t)pop_state & 7u))
     return fail(DQLB200_ERR_ARG, "misaligned buffer (env_state needs 16 B, pop_state 8 B)");
+  // The packed env state counts an episode's steps in STEP_BITS bits and the goal steps in CC_BITS bits (env_state.cuh); a count
+  // that reaches the limit ends the episode and is never stored, so the limit itself may be the largest field value.  (The
+  // single-object facade kernels keep their counts in float64 and never bind an env state: any t_max * f_ag works there.)
+  constexpr int max_steps = (1 << dql::STEP_BITS) - 1, max_goal = (1 << dql::CC_BITS) - 1;
+  if (h->cfg.timeout_steps > max_steps)
+    return fail(DQLB200_ERR_ARG, "episode length timeout_steps = " + std::to_string(h->cfg.timeout_steps) + " (t_max * f_ag = " +
+                                     std::to_string(h->cfg.timeout_threshold) + ") exceeds " + std::to_string(max_steps) +
+                                     ", the largest step count the env state holds");
+  if (h->cfg.success_steps > max_goal)
+    return fail(DQLB200_ERR_ARG, "goal length success_steps = " + std::to_string(h->cfg.success_steps) + " (f_ag = " +
+                                     std::to_string(h->cfg.f_ag) + ") exceeds " + std::to_string(max_goal) +
+                                     ", the largest goal-step count the env state holds");
   h->env_state = env_state;
   h->tables = tables;
   h->pop_state = pop_state;

@@ -91,8 +91,10 @@ typedef struct dqlb200_config {
   float angle_cut[6];               /* first pitch whose argmin index is >= i+1 (PKG/mdp.py:318-323) */
   float fz_lo, fz_hi;               /* fly zone x: out  <=>  !(x >= fz_lo) || (x >= fz_hi)  (PKG/mdp.py:365-368) */
   float z_min_cut, z_max_cut;       /* z < minimum_altitude <=> !(z >= z_min_cut); z > p_max <=> z >= z_max_cut */
-  int32_t timeout_steps;            /* first integer n with n >= t_max * f_ag   (459) */
-  int32_t success_steps;            /* first integer n with n >= f_ag           (23)  */
+  int32_t timeout_steps;            /* first integer n with n >= t_max * f_ag   (459); <= 511 to bind an env state */
+  int32_t success_steps;            /* first integer n with n >= f_ag           (23);  <= 31 to bind an env state  */
+  /* The env state packs the step count into 9 bits and the goal-step count into 5 (csrc/env_state.cuh): dqlb200_bind refuses
+   * (DQLB200_ERR_ARG) a configuration whose counts would overflow them.  The facade kernels count in float64 and have no limit. */
   dqlb200_reward_level reward[DQLB200_MAX_CURRICULUM];
   double p_max, v_max, theta_max, delta_theta, w_p, w_v, w_theta;
   /* float64 tables for the facade kernel, which discretises arbitrary float64 observations with the
@@ -261,7 +263,8 @@ int dqlb200_config_is_default(const dqlb200_config* cfg);
  *   tables    : [n_populations][3][DQLB200_MAX_CELLS] 32-bit words: Q_a (f32), Q_b (f32), count (u32)
  *               == DoubleQLearningAgent.Q_table_a / Q_table_b / state_action_counter, row-major
  *               (curriculum, p, v, a, theta, action) like the .npy files (PKG/double_q_learning.py:38-53)
- *   pop_state : n_populations x dqlb200_population_state */
+ *   pop_state : n_populations x dqlb200_population_state
+ * Refused (DQLB200_ERR_ARG) when timeout_steps > 511 or success_steps > 31: the env state cannot count such episodes. */
 int dqlb200_bind(dqlb200_handle* h, void* env_state, void* tables, void* pop_state);
 
 /* Borrow the per-env state of the acceleration estimator (accel_mode != 0): n_populations * envs_per_population x 16 bytes

@@ -51,15 +51,15 @@ def exploration_rate(episode: int, w: int) -> float:
     return max(1 + (0.01 - 1) * (episode - 800) / (2000 - 800), 0.01)
 
 
-SCALE_MODIFICATION = [0.8172650252856599, 0.8211253690681617, 0.8257273369742982, 0.8311571820651724]
+SCALE_MODIFICATION = (0.8172650252856599, 0.8211253690681617, 0.8257273369742982, 0.8311571820651724)
 
 
-def transfer_ratio(step: int) -> float:
-    """PKG/trainer.py:128-138."""
+def transfer_ratio(step: int, scale: Sequence[float] = SCALE_MODIFICATION) -> float:
+    """PKG/trainer.py:128-138 (``scale`` = Trainer's scale_modification_value)."""
     if step < 1:
         return 1.0
-    if step < len(SCALE_MODIFICATION) + 1:
-        return SCALE_MODIFICATION[step - 1]
+    if step < len(scale) + 1:
+        return scale[step - 1]
     raise ValueError(f"Transfer learning can be done up to the 5th curriculum step, {step} is invalid")
 
 

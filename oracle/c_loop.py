@@ -88,7 +88,7 @@ def run_population_c(n_envs: int, n_steps: int, seed: int = 42, population: int 
     lp = LoopParams(dz=d.dz, z_touch=d.z_touch, half_platform=d.half_platform, p_max_f=d.p_max, two_p_max_f=d.two_p_max, sigma_x=d.sigma_x,
                     f_ag=tp.f_ag, t_max=tp.t_max, p_max=tp.p_max, alpha_min=tp.alpha_min, omega=tp.omega, gamma=tp.gamma)
     tpc = TrainerParamsC(tp.curriculum_steps, tp.successive_successful_episodes, {"reference": 0, "paper": 1}[tp.transfer_mode],
-                         tp.success_rate, tp.max_num_episodes, (C.c_float * 5)(*[np.float32(transfer_ratio(k)) for k in range(5)]))
+                         tp.success_rate, tp.max_num_episodes, (C.c_float * 5)(*[np.float32(transfer_ratio(k, tp.scale_modification_value)) for k in range(5)]))
     qa = np.zeros(2835, np.float32) if qa0 is None else np.ascontiguousarray(qa0, np.float32).reshape(-1).copy()
     qb = np.zeros(2835, np.float32) if qb0 is None else np.ascontiguousarray(qb0, np.float32).reshape(-1).copy()
     count = np.zeros(2835, np.float64)

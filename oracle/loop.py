@@ -22,12 +22,12 @@ from __future__ import annotations
 
 from collections import deque
 from dataclasses import dataclass, field
-from typing import Optional
+from typing import Optional, Tuple
 
 import numpy as np
 
 from . import philox
-from .agent_oracle import AgentOracle, exploration_rate, explore_threshold, state_id, transfer_ratio
+from .agent_oracle import SCALE_MODIFICATION, AgentOracle, exploration_rate, explore_threshold, state_id, transfer_ratio
 from .dynamics import StandInDet, StandInParams, add_observation_noise
 from .mdp_oracle import (MdpParams, TERMINAL_SUCCESS, TrainingMdpOracle)
 
@@ -46,6 +46,7 @@ class TrainerParams:
     f_ag: float = 22.92
     p_max: float = 4.5
     transfer_mode: str = "reference"      # "reference" (quirk Q7) | "paper"
+    scale_modification_value: Tuple[float, ...] = SCALE_MODIFICATION     # transfer ratios of steps 1..4
 
 
 class PopulationOracle:
@@ -164,9 +165,9 @@ class PopulationOracle:
             self.window.clear()
         self.promotions.append((self.t, self.w, promoted))
         if tp.transfer_mode == "reference":
-            ag.transfer(self.w, transfer_ratio(self.w))
+            ag.transfer(self.w, transfer_ratio(self.w, tp.scale_modification_value))
         elif self.w + 1 < tp.curriculum_steps:
-            ag.transfer(self.w + 1, transfer_ratio(self.w + 1))
+            ag.transfer(self.w + 1, transfer_ratio(self.w + 1, tp.scale_modification_value))
         self.w += 1
         self.episodes_done = 0
         if self.w >= tp.curriculum_steps:
