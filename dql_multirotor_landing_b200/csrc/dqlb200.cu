@@ -10,7 +10,8 @@
 //                        reward, learning rate (R11), table update (R12), auto-reset, success window / promotion /
 //                        transfer (R13/R14).  Q_a / count live in shared memory for the whole launch.
 //   env_kernels.cuh      reset_kernel (R1 + R8 for every env), eval_kernel / eval2d_kernel (R15: greedy SimulationMdp
-//                        episodes, one thread per episode, one or two axes), env_reset_kernel / env_step_kernel (gym surface)
+//                        episodes, one thread per episode, one or two axes), eval_agents_kernel (every agent's greedy policy
+//                        from its live tables, one launch), env_reset_kernel / env_step_kernel (gym surface)
 //   facade_kernels.cuh   float64 single-object TrainingMdp / SimulationMdp / DoubleQLearningAgent calls, division self-test
 //   table_kernels.cuh    transfer (R13), shared-table pack/apply, replica merge, atomic-roof micro-benchmark
 //
@@ -484,6 +485,32 @@ int dqlb200_eval_greedy(dqlb200_handle* h, int population, const uint8_t* policy
   else
     dql::eval_kernel<true><<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(h->kc, h->d_pop_params, population, policy, first_episode, n_episodes,
                                                                              working_step, (dqlb200_eval_stats*)stats_out, tr, trace ? trace_steps : 0);
+  CUDA_TRY(cudaGetLastError());
+  return DQLB200_OK;
+}
+
+int dqlb200_eval_agents(dqlb200_handle* h, int working_step, int64_t first_episode, int64_t episodes_per_agent, void* stats_out,
+                        uint8_t* policy_out, void* stream) {
+  if (!h) return fail(DQLB200_ERR_ARG, "null handle");
+  if (!stats_out) return fail(DQLB200_ERR_ARG, "stats_out required");
+  if (working_step < -1 || working_step >= h->cfg.curriculum_steps)
+    return fail(DQLB200_ERR_ARG, "working_step must be -1 (each agent's live step) or 0 .. curriculum_steps - 1");
+  if (!h->tables || !h->pop_state) return fail(DQLB200_ERR_STATE, "tables / trainer state not bound");
+  DQL_NEED_FILTER(h);
+  if (episodes_per_agent <= 0) return DQLB200_OK;
+  const long long blocks_per_agent = (episodes_per_agent + 255) / 256;
+  const int R = h->cfg.replicas_per_population, n_agents = h->cfg.n_populations / R;
+  if (blocks_per_agent * n_agents > 0x7FFFFFFFLL) return fail(DQLB200_ERR_ARG, "episodes_per_agent * n_agents exceeds one launch's grid");
+  CUDA_TRY(cudaSetDevice(h->device));
+  const unsigned grid = (unsigned)(blocks_per_agent * n_agents);
+  cudaStream_t s = (cudaStream_t)stream;
+  const auto* ps = (const dqlb200_population_state*)h->pop_state;
+  if (h->kc_default)
+    dql::eval_agents_kernel<false><<<grid, 256, 0, s>>>(h->kc, h->d_pop_params, (const uint32_t*)h->tables, ps, R, (int)blocks_per_agent,
+                                                       first_episode, episodes_per_agent, working_step, (dqlb200_eval_stats*)stats_out, policy_out);
+  else
+    dql::eval_agents_kernel<true><<<grid, 256, 0, s>>>(h->kc, h->d_pop_params, (const uint32_t*)h->tables, ps, R, (int)blocks_per_agent,
+                                                      first_episode, episodes_per_agent, working_step, (dqlb200_eval_stats*)stats_out, policy_out);
   CUDA_TRY(cudaGetLastError());
   return DQLB200_OK;
 }

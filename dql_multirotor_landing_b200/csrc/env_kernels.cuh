@@ -34,6 +34,53 @@ __global__ void reset_kernel(const __grid_constant__ KC kc, EnvPtrs env, dqlb200
 // -------------------------------------------------------------------------------------------------
 // R15: greedy evaluation, SimulationMdp semantics (PKG/mdp.py:784-886, scripts/simulation.py:48-63)
 // -------------------------------------------------------------------------------------------------
+// One greedy episode of `policy` (a shared-memory LUT): the reset draw of episode `ep`, the SimulationMdp check chain, and the
+// optional per-step trace (row `i` of arrays [trace_steps][n_episodes]).  Returns the termination code; `step` = its length.
+template <bool GENERIC, class KT>
+__device__ __forceinline__ int greedy_episode(const KT& kk, const dqlb200_population_params& pp, const dqlb200_cuts& cuts,
+                                              const uint8_t* s_policy, unsigned long long ep, const dqlb200_trace& trace,
+                                              int trace_steps, long long i, long long n_episodes, int& step) {
+  const uint4 d = philox4x32_10(make_uint4((uint32_t)ep, 0u, PURPOSE_RESET, pp.population_id), pp.seed_lo, pp.seed_hi);
+  Body b;
+  Kf kf = kf_initial();       // accel_mode != 0: every evaluation episode runs on a freshly started simulator
+  Kf* const kfp = (GENERIC && kk.accel_mode != 0) ? &kf : nullptr;
+  Ext ex = ext_initial(kk);
+  Ext* const exp_ = (GENERIC && kk.dynamics_model != 0) ? &ex : nullptr;
+  Obs o = dyn_reset(kk, pp, b, d, /*normal_init=*/false, /*simulation=*/true, kk.dz_sim, kfp, exp_);
+  uint32_t sid = (uint32_t)discretise_cuts(cuts, kk.angle_cut, o).id();
+  double sp = 0.0;
+  int code = DQLB200_NON_TERMINAL;
+  step = 0;
+  while (code < DQLB200_TERMINAL_SUCCESS) {
+    const int a = s_policy[sid];
+    sp = apply_action(kk, sp, a);
+    dyn_advance(kk, pp, b, (float)sp, kfp, exp_, kk.vz_sim);
+    step += 1;
+    o = dyn_observe(kk, pp, b, step, kk.dz_sim, kfp, exp_);
+    const uint32_t sid2 = (uint32_t)discretise_cuts(cuts, kk.angle_cut, o).id();
+    if (o.contact) code = DQLB200_TERMINAL_CONTACT;
+    else if (!(o.rel_p >= kk.fz_lo) || (o.rel_p >= kk.fz_hi)) code = DQLB200_TERMINAL_FLYZONE_X;
+    else if (!(o.z >= kk.z_min_cut)) code = DQLB200_TERMINAL_MINIMUM_ALTITUDE;
+    else if (o.z >= kk.z_max_cut) code = DQLB200_TERMINAL_FLYZONE_Z;
+    else if (step >= kk.timeout_steps) code = DQLB200_TERMINAL_TIMEOUT;
+    if (step <= trace_steps) {
+      const size_t ti = (size_t)(step - 1) * (size_t)n_episodes + (size_t)i;
+      if (trace.obs) {
+        float* po = trace.obs + ti * 5;
+        po[0] = o.rel_p; po[1] = o.rel_v; po[2] = o.rel_a; po[3] = o.pitch; po[4] = o.z;
+      }
+      if (trace.action) trace.action[ti] = (uint8_t)a;
+      if (trace.code) trace.code[ti] = (uint8_t)code;
+      if (trace.done) trace.done[ti] = (uint8_t)(code >= DQLB200_TERMINAL_SUCCESS);
+      if (trace.contact) trace.contact[ti] = (uint8_t)o.contact;
+      if (trace.state) trace.state[ti] = (uint16_t)sid;
+      if (trace.next_state) trace.next_state[ti] = (uint16_t)sid2;
+    }
+    sid = sid2;
+  }
+  return code;
+}
+
 template <bool GENERIC>
 __global__ void __launch_bounds__(256) eval_kernel(const __grid_constant__ KC kc, const dqlb200_population_params* pop_params,
                                                    int population, const uint8_t* __restrict__ policy,
@@ -50,45 +97,8 @@ __global__ void __launch_bounds__(256) eval_kernel(const __grid_constant__ KC kc
   const dqlb200_population_params pp = pop_params[population];
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n_episodes) {
-    const unsigned long long ep = (unsigned long long)(first_episode + i);
-    const uint4 d = philox4x32_10(make_uint4((uint32_t)ep, 0u, PURPOSE_RESET, pp.population_id), pp.seed_lo, pp.seed_hi);
-    Body b;
-    Kf kf = kf_initial();       // accel_mode != 0: every evaluation episode runs on a freshly started simulator
-    Kf* const kfp = (GENERIC && kk.accel_mode != 0) ? &kf : nullptr;
-    Ext ex = ext_initial(kk);
-    Ext* const exp_ = (GENERIC && kk.dynamics_model != 0) ? &ex : nullptr;
-    Obs o = dyn_reset(kk, pp, b, d, /*normal_init=*/false, /*simulation=*/true, kk.dz_sim, kfp, exp_);
-    uint32_t sid = (uint32_t)discretise_cuts(cuts, kk.angle_cut, o).id();
-    double sp = 0.0;
-    int code = DQLB200_NON_TERMINAL;
-    int step = 0;
-    while (code < DQLB200_TERMINAL_SUCCESS) {
-      const int a = s_policy[sid];
-      sp = apply_action(kk, sp, a);
-      dyn_advance(kk, pp, b, (float)sp, kfp, exp_, kk.vz_sim);
-      step += 1;
-      o = dyn_observe(kk, pp, b, step, kk.dz_sim, kfp, exp_);
-      const uint32_t sid2 = (uint32_t)discretise_cuts(cuts, kk.angle_cut, o).id();
-      if (o.contact) code = DQLB200_TERMINAL_CONTACT;
-      else if (!(o.rel_p >= kk.fz_lo) || (o.rel_p >= kk.fz_hi)) code = DQLB200_TERMINAL_FLYZONE_X;
-      else if (!(o.z >= kk.z_min_cut)) code = DQLB200_TERMINAL_MINIMUM_ALTITUDE;
-      else if (o.z >= kk.z_max_cut) code = DQLB200_TERMINAL_FLYZONE_Z;
-      else if (step >= kk.timeout_steps) code = DQLB200_TERMINAL_TIMEOUT;
-      if (step <= trace_steps) {
-        const size_t ti = (size_t)(step - 1) * (size_t)n_episodes + (size_t)i;
-        if (trace.obs) {
-          float* po = trace.obs + ti * 5;
-          po[0] = o.rel_p; po[1] = o.rel_v; po[2] = o.rel_a; po[3] = o.pitch; po[4] = o.z;
-        }
-        if (trace.action) trace.action[ti] = (uint8_t)a;
-        if (trace.code) trace.code[ti] = (uint8_t)code;
-        if (trace.done) trace.done[ti] = (uint8_t)(code >= DQLB200_TERMINAL_SUCCESS);
-        if (trace.contact) trace.contact[ti] = (uint8_t)o.contact;
-        if (trace.state) trace.state[ti] = (uint16_t)sid;
-        if (trace.next_state) trace.next_state[ti] = (uint16_t)sid2;
-      }
-      sid = sid2;
-    }
+    int step;
+    const int code = greedy_episode<GENERIC>(kk, pp, cuts, s_policy, (unsigned long long)(first_episode + i), trace, trace_steps, i, n_episodes, step);
     atomicAdd(&s_hist[code], 1u);
     atomicAdd(&s_steps, (unsigned int)step);
     atomicAdd(&s_eps, 1u);
@@ -98,6 +108,69 @@ __global__ void __launch_bounds__(256) eval_kernel(const __grid_constant__ KC kc
   if (threadIdx.x == 0) {
     atomicAdd((unsigned long long*)&stats->steps, (unsigned long long)s_steps);
     atomicAdd((unsigned long long*)&stats->episodes, (unsigned long long)s_eps);
+  }
+}
+
+// Greedy action of state s from float32 tables: the first maximum of (Q_a + Q_b) * 0.5f over the actions in order, each operation
+// rounded to nearest -- the arithmetic of build_snapshot (train_kernel) and agent_select_kernel.
+__device__ __forceinline__ uint8_t greedy_action_f32(const float* __restrict__ qa, const float* __restrict__ qb, int s) {
+  const float p0 = fmul(fadd(qa[s * 3 + 0], qb[s * 3 + 0]), 0.5f);
+  const float p1 = fmul(fadd(qa[s * 3 + 1], qb[s * 3 + 1]), 0.5f);
+  const float p2 = fmul(fadd(qa[s * 3 + 2], qb[s * 3 + 2]), 0.5f);
+  int a = 0;
+  float best = p0;
+  if (p1 > best) { best = p1; a = 1; }
+  if (p2 > best) { a = 2; }
+  return (uint8_t)a;
+}
+
+// Every agent's greedy policy in one launch: blocks_per_agent blocks of 256 episodes per agent on a flat 1-D grid (agent =
+// blockIdx.x / blocks_per_agent).  Agent g reads replica g * replicas: its tables (the LUT is built per block in shared memory),
+// Philox key, platform and -- for w < 0 -- its live working step.  Episode i of agent g is episode first_episode + i of
+// eval_kernel for population g * replicas under the same LUT.  Reads the tables and trainer state, writes only stats / policy_out.
+template <bool GENERIC>
+__global__ void __launch_bounds__(256) eval_agents_kernel(const __grid_constant__ KC kc, const dqlb200_population_params* pop_params,
+                                                          const uint32_t* __restrict__ tables, const dqlb200_population_state* __restrict__ pop_state,
+                                                          int replicas, int blocks_per_agent, long long first_episode,
+                                                          long long episodes_per_agent, int w, dqlb200_eval_stats* stats,
+                                                          uint8_t* __restrict__ policy_out) {
+  const auto& kk = ConstsOf<GENERIC>::get(kc);
+  constexpr int N_STATES = DQLB200_MAX_CURRICULUM * DQLB200_STATES_PER_LEVEL;
+  __shared__ uint8_t s_policy[N_STATES];
+  __shared__ dqlb200_cuts cuts;
+  __shared__ unsigned int s_hist[9], s_steps, s_eps;
+  const int agent = (int)(blockIdx.x / (unsigned)blocks_per_agent);
+  const int block_in_agent = (int)(blockIdx.x - (unsigned)agent * (unsigned)blocks_per_agent);
+  const int pop = agent * replicas;
+  const float* qa = reinterpret_cast<const float*>(tables + (size_t)pop * 3 * DQLB200_MAX_CELLS);
+  const float* qb = qa + DQLB200_MAX_CELLS;
+  const int live_states = kc.curriculum_steps * DQLB200_STATES_PER_LEVEL;
+  for (int s = threadIdx.x; s < N_STATES; s += blockDim.x) s_policy[s] = s < live_states ? greedy_action_f32(qa, qb, s) : (uint8_t)0;
+  if (threadIdx.x == 0) {
+    const int wl = w >= 0 ? w : min(max(pop_state[pop].working_step, 0), kc.curriculum_steps - 1);      // clamped: never index past cuts[]
+    cuts = kc.cuts[wl];
+    s_steps = s_eps = 0u;
+  }
+  if (threadIdx.x < 9) s_hist[threadIdx.x] = 0u;
+  __syncthreads();
+  if (policy_out && block_in_agent == 0)
+    for (int s = threadIdx.x; s < N_STATES; s += blockDim.x) policy_out[(size_t)agent * N_STATES + s] = s_policy[s];
+  const dqlb200_population_params pp = pop_params[pop];
+  const long long i = (long long)block_in_agent * blockDim.x + threadIdx.x;
+  if (i < episodes_per_agent) {
+    int step;
+    const dqlb200_trace no_trace = {};
+    const int code = greedy_episode<GENERIC>(kk, pp, cuts, s_policy, (unsigned long long)(first_episode + i), no_trace, 0, i, episodes_per_agent, step);
+    atomicAdd(&s_hist[code], 1u);
+    atomicAdd(&s_steps, (unsigned int)step);
+    atomicAdd(&s_eps, 1u);
+  }
+  __syncthreads();
+  dqlb200_eval_stats* st = stats + agent;
+  if (threadIdx.x < 9 && s_hist[threadIdx.x]) atomicAdd((unsigned long long*)&st->termination_hist[threadIdx.x], (unsigned long long)s_hist[threadIdx.x]);
+  if (threadIdx.x == 0) {
+    atomicAdd((unsigned long long*)&st->steps, (unsigned long long)s_steps);
+    atomicAdd((unsigned long long*)&st->episodes, (unsigned long long)s_eps);
   }
 }
 

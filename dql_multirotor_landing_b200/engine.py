@@ -305,6 +305,29 @@ class Engine:
         torch.cuda.synchronize(dev)
         return _eval_result(K.EvalStats.from_buffer_copy(stats.cpu().numpy().tobytes()), out)
 
+    def eval_agents(self, episodes_per_agent: int, *, working_step: Optional[int] = None, first_episode: int = 0,
+                    return_policies: bool = False) -> dict:
+        """Greedy SimulationMdp episodes of every agent's current policy, built on the device from the live float32 tables
+        (dqlb200_eval_agents): one launch, one copy back, one synchronisation.  Agent g is replica group g (population g * R);
+        working_step None = each agent's live working step.  Agent g's episodes are those of
+        eval_greedy(<its float32 greedy LUT>, episodes_per_agent, population=g * R, first_episode=..., working_step=...).
+        Returns NumPy arrays over the agents: episodes [A], steps [A], termination_hist [A, 9], success_rate [A] (goal or
+        contact, the reference's two "SUCCESS" codes) and, with return_policies, policy [A, 945] uint8."""
+        A = self.P // self.R
+        stats_bytes, n_states = A * C.sizeof(K.EvalStats), K.MAX_CURRICULUM * K.STATES_PER_LEVEL
+        buf = torch.zeros(stats_bytes + (A * n_states if return_policies else 0), dtype=torch.uint8, device=self.device)
+        w = -1 if working_step is None else int(working_step)
+        _ffi.check(self.lib.dqlb200_eval_agents(self.handle, w, int(first_episode), int(episodes_per_agent), buf.data_ptr(),
+                                                buf.data_ptr() + stats_bytes if return_policies else None, self._stream()))
+        host = buf.cpu().numpy()          # synchronises the stream
+        st = host[:stats_bytes].view(np.uint64).reshape(A, 11).astype(np.int64)
+        res = dict(episodes=st[:, 0], steps=st[:, 1], termination_hist=st[:, 2:])
+        hist = res["termination_hist"]            # codes 2 (goal) and 3 (contact); a SimulationMdp episode only ends in 3
+        res["success_rate"] = (hist[:, 2] + hist[:, 3]) / np.maximum(res["episodes"], 1)
+        if return_policies:
+            res["policy"] = host[stats_bytes:].reshape(A, n_states).copy()
+        return res
+
     def eval_greedy_2d(self, policy_x: np.ndarray, policy_y: np.ndarray, n_episodes: int, *, two_axis: Optional[K.TwoAxisParameters] = None,
                        seed: int = 42, stream_id: int = 0, first_episode: int = 0, working_step: int = 4, trace_steps: int = 0):
         """Greedy two-axis SimulationMdp episodes: agent_x and agent_y both predict every step (scripts/simulation.py:48-63).

@@ -45,6 +45,9 @@ def replica_shape(num_envs: int, merge_every: int = 1) -> int:
 
 
 class Trainer:
+    _eval_every: Optional[int] = None       # greedy evaluation of every agent after each `eval_every`-th chunk (None: off)
+    _eval_episodes: int = 1024
+
     def __init__(
         self,
         curriculum_steps: int = 5,
@@ -79,6 +82,8 @@ class Trainer:
         tensorboard: bool = False,
         verbose: bool = True,
         direction: str = "x",
+        eval_every: Optional[int] = None,
+        eval_episodes: int = 1024,
     ) -> None:
         np.random.seed(seed)                                        # PKG/trainer.py:45
         if not double_q_learning_agent:
@@ -119,6 +124,10 @@ class Trainer:
         if direction not in ("x", "y"):
             raise ValueError("direction must be 'x' or 'y' (training.launch direction:=x|y, training_x.sh / training_y.sh)")
         self._direction = direction
+        if eval_every is not None:          # set only when asked for, so a default Trainer pickles exactly as before
+            if eval_every < 1 or eval_episodes < 1:
+                raise ValueError("eval_every and eval_episodes must be >= 1")
+            self._eval_every, self._eval_episodes = eval_every, eval_episodes
         self._engine = None
         self.history = []             # one dict per chunk (population 0)
 
@@ -216,7 +225,7 @@ class Trainer:
         eng.reset(self._working_curriculum_step)
         info: Dict[str, Any] = {}
         prev = eng.population_state()
-        global_steps = 0
+        global_steps = chunks = 0
         while True:
             if self._replicas > 1:
                 eng.train_merged(self._chunk_steps, self._merge_every)
@@ -224,6 +233,7 @@ class Trainer:
                 eng.train(self._chunk_steps)
             eng.check_errors()
             global_steps += self._chunk_steps
+            chunks += 1
             ps = eng.population_state()
             p0 = ps[0]
             self._working_curriculum_step = int(p0["working_step"])
@@ -247,7 +257,12 @@ class Trainer:
                 "Global steps": int(p0["t"]), "Env steps": int(ps["total_steps"].sum()), "Episodes in chunk": d_ep,
                 "Pooled episodes": pooled_episodes,
             }
-            self.history.append(dict(info, working_step=self._working_curriculum_step))
+            entry = {}
+            if self._eval_every is not None and chunks % self._eval_every == 0:
+                rates = eng.eval_agents(self._eval_episodes)["success_rate"]      # greedy policies at the live working steps
+                info["Greedy success rate"] = float(rates[0])
+                entry["Greedy success rates"] = [float(r) for r in rates]
+            self.history.append(dict(info, working_step=self._working_curriculum_step, **entry))
             if len(self.history) > 2048:          # bounded: the history is pickled with every checkpoint
                 del self.history[:1024]
             advanced = any(int(ps[p]["working_step"]) != int(prev[p]["working_step"]) or int(ps[p]["finished"]) != int(prev[p]["finished"])
@@ -278,6 +293,8 @@ class Trainer:
             writer.add_scalar("Episode/Exploration Rate", info["Exploration rate"], step)
             writer.add_scalar("Episode/Learning Rate", info["Learning rate"], step)
             writer.add_scalar("Episode/Mean reward", info["Mean reward"], step)
+            if "Greedy success rate" in info:
+                writer.add_scalar("Episode/Greedy Success Rate", info["Greedy success rate"], step)
             writer.add_text("Episode/Termination Condition", info["Termination condition"], step)
             writer.close()
         if clean:

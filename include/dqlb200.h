@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define DQLB200_ABI_VERSION 8
+#define DQLB200_ABI_VERSION 9
 #define DQLB200_MAX_CURRICULUM 5
 #define DQLB200_STATES_PER_LEVEL 189          /* 3*3*3*7      (PKG/double_q_learning.py:38-40) */
 #define DQLB200_CELLS_PER_LEVEL 567           /* 189 * 3 actions */
@@ -316,6 +316,31 @@ int dqlb200_train_host_ext(dqlb200_handle* h, int k_steps, void* env_state_host,
 int dqlb200_eval_greedy(dqlb200_handle* h, int population, const uint8_t* policy, int64_t first_episode,
                         int64_t n_episodes, int working_step, void* stats_out, const dqlb200_trace* trace,
                         int trace_steps, void* stream);
+
+/* Greedy SimulationMdp episodes of EVERY agent's current policy, built on the device from the bound float32 tables, in one
+ * launch and without a host round trip per agent.
+ *   agents       : agent g is the replica group g*R .. g*R+R-1 (R = replicas_per_population; R = 1: every population is an
+ *                  agent), n_agents = n_populations / R.  The group is read through replica g*R: its tables, its
+ *                  dqlb200_population_params (Philox key, population_id, platform, axis) and its trainer state.
+ *                  dqlb200_train_merged and dqlb200_replica_merge leave all replicas of a group identical; between merges the
+ *                  other replicas are not looked at.
+ *   policy       : for every state s < curriculum_steps * 189 the FIRST maximum over a of float32 (Q_a[s,a] + Q_b[s,a]) * 0.5f,
+ *                  each operation rounded to nearest (the arithmetic of the greedy action in dqlb200_train and
+ *                  dqlb200_agent_select, i.e. the policy the agent follows at epsilon = 0); states at and above
+ *                  curriculum_steps * 189 act 0.
+ *   working_step : w >= 0 evaluates every agent under the cut table of step w; -1 uses each agent's live
+ *                  dqlb200_population_state.working_step (read on the device; a finished agent holds curriculum_steps - 1).
+ *   episodes     : episode i of agent g uses the reset draw (first_episode + i, 0, reset, population_id) under the Philox key of
+ *                  replica g*R, so agent g's episodes are, one for one, those of dqlb200_eval_greedy(population = g*R, policy =
+ *                  its float32 LUT, first_episode, n_episodes = episodes_per_agent, working_step = w).  With accel_mode /
+ *                  dynamics_model every episode starts a fresh simulator, as there.
+ *   stats_out    : device dqlb200_eval_stats[n_agents], accumulated (the caller zeroes), exact integer counts.
+ *   policy_out   : nullable, device uint8 [n_agents][DQLB200_MAX_CURRICULUM * DQLB200_STATES_PER_LEVEL]: the LUT evaluated.
+ * Nothing bound is written: env state, tables, trainer state and the option buffers are only read (or not read at all).
+ * Refused: working_step < -1 or >= curriculum_steps, stats_out NULL (DQLB200_ERR_ARG); tables or trainer state not bound, an
+ * option without its bound buffer (DQLB200_ERR_STATE).  episodes_per_agent <= 0 does nothing. */
+int dqlb200_eval_agents(dqlb200_handle* h, int working_step, int64_t first_episode, int64_t episodes_per_agent,
+                        void* stats_out, uint8_t* policy_out, void* stream);
 
 /* Un-fused environment entry points: the gym surface of the reference with caller-supplied actions, no agent, no table.
  *   dqlb200_env_reset  replaces TrainingLandingEnv.reset / SimulationLandingEnv.reset (PKG/landing_simulation_env.py:167-243,

@@ -3,6 +3,7 @@ training_y.sh -> launch/training.launch): no ROS node, no Gazebo; the batched Tr
 
     python scripts/training.py                       # x axis, 4 096 envs on one table pair
     python scripts/training.py --direction y --num-envs 65536 --success-rate 0.8
+    python scripts/training.py --eval-every 10       # + greedy success rate of the live policy every 10 chunks
 """
 import argparse
 import pathlib
@@ -25,12 +26,15 @@ if __name__ == "__main__":
     ap.add_argument("--noise", action="store_true", help="manager_node's default observation noise (0.25 m, 0.1 m/s)")
     ap.add_argument("--kalman", action="store_true", help="the observation node's Kalman-filtered acceleration estimate")
     ap.add_argument("--second-order", action="store_true", help="second-order attitude + vertical PID dynamics")
+    ap.add_argument("--eval-every", type=int, default=None, metavar="N",
+                    help="log the greedy policy's SimulationMdp success rate after every N-th chunk (off by default)")
     a = ap.parse_args()
     dp = K.DynamicsParameters(n_sub=4 if (a.kalman or a.second_order) else 1,
                               noise_pos_sd=0.25 if a.noise else 0.0, noise_vel_sd=0.1 if a.noise else 0.0,
                               accel_mode="kalman_reference" if a.kalman else "exact",
                               dynamics_model="second_order" if a.second_order else "first_order")
     trainer = Trainer(seed=a.seed, success_rate=a.success_rate, save_path=a.save_path, num_envs=a.num_envs, device=a.device,
-                      direction=a.direction, max_global_steps=a.max_global_steps, dynamics=dp)
+                      direction=a.direction, max_global_steps=a.max_global_steps, dynamics=dp,
+                      eval_every=a.eval_every)
     info = trainer.curriculum_training()
     trainer.log(info, clean=False)

@@ -1,5 +1,6 @@
 """Learning-quality probe (development aid; SURVEY.md A.4 behavioural golden): success rate per chunk of training at curriculum
-step 0, promotion off.  One script for the cases DESIGN.md section 3 quotes:
+step 0, promotion off; beside it the greedy success rate of the agents' live policies (SimulationMdp, 1,024 episodes per agent,
+Engine.eval_agents).  One script for the cases DESIGN.md section 3 quotes:
 
     python tools/learn_probe.py single               one env / 64 / 1,024 envs per CTA (S1 semantics), 8 seeds each
     python tools/learn_probe.py merge                one agent as R replicas x 128 envs, merge interval 1 / 8 / 64
@@ -38,8 +39,10 @@ def run(R, n_r, merge_every, total_steps, v_mp=1.6, chunks=6, n_sub=1):
         ep, su = int(ps["total_episodes"].sum()), int(ps["total_successes"].sum())
         hist = ps["termination_hist"].sum(axis=0).astype(float)
         dh = hist - prev_hist
+        greedy = float(eng.eval_agents(1024)["success_rate"].mean())      # greedy policies, SimulationMdp, at the live working step
         rows.append(dict(global_steps=done, episodes_per_env=ep // (P * n_r), success_rate_in_chunk=round((su - prev_su) / max(ep - prev_ep, 1), 3),
-                         share_success_flyzone_timeout=[round(x, 3) for x in (dh / max(dh.sum(), 1))[[2, 4, 8]]]))
+                         share_success_flyzone_timeout=[round(x, 3) for x in (dh / max(dh.sum(), 1))[[2, 4, 8]]],
+                         greedy_success_rate=round(greedy, 3)))
         prev_ep, prev_su, prev_hist = ep, su, hist
     print(json.dumps(dict(replicas=R, envs_per_cta=n_r, merge_every=merge_every if R > 0 else None, v_mp=v_mp, n_sub=n_sub, curve=rows)), flush=True)
     eng.close()
