@@ -16,7 +16,7 @@ SYMBOLS = [
     "dqlb200_abi_version", "dqlb200_config_bytes", "dqlb200_population_state_bytes", "dqlb200_last_error",
     "dqlb200_termination_string", "dqlb200_create", "dqlb200_destroy", "dqlb200_bind", "dqlb200_reset",
     "dqlb200_train", "dqlb200_train_host", "dqlb200_train_host_ext", "dqlb200_eval_greedy", "dqlb200_transfer", "dqlb200_check_errors",
-    "dqlb200_shared_pack", "dqlb200_shared_apply", "dqlb200_mdp_facade_step", "dqlb200_agent_facade", "dqlb200_selftest_division", "dqlb200_replica_merge", "dqlb200_bind_merge_snapshot", "dqlb200_eval_greedy_2d", "dqlb200_eval2d_params_bytes", "dqlb200_bench_table_rmw", "dqlb200_train_merged", "dqlb200_env_reset", "dqlb200_env_step", "dqlb200_agent_select", "dqlb200_agent_update", "dqlb200_uses_default_instance", "dqlb200_config_is_default", "dqlb200_bench_launch_floor", "dqlb200_bind_filter_state", "dqlb200_bind_dynamics_state", "dqlb200_selftest_discretise", "dqlb200_env_state_bytes", "dqlb200_shared_sync_nccl", "dqlb200_eval_agents",
+    "dqlb200_shared_pack", "dqlb200_shared_apply", "dqlb200_mdp_facade_step", "dqlb200_agent_facade", "dqlb200_selftest_division", "dqlb200_replica_merge", "dqlb200_bind_merge_snapshot", "dqlb200_eval_greedy_2d", "dqlb200_eval2d_params_bytes", "dqlb200_bench_table_rmw", "dqlb200_train_merged", "dqlb200_env_reset", "dqlb200_env_step", "dqlb200_agent_select", "dqlb200_agent_update", "dqlb200_uses_default_instance", "dqlb200_config_is_default", "dqlb200_bench_launch_floor", "dqlb200_bind_filter_state", "dqlb200_bind_dynamics_state", "dqlb200_selftest_discretise", "dqlb200_env_state_bytes", "dqlb200_shared_sync_nccl", "dqlb200_eval_agents", "dqlb200_eval_pairs",
 ]
 
 OP_ACTION, OP_OBSERVE, OP_CHECK, OP_REWARD, OP_RESET, OP_SIMULATION = 1, 2, 4, 8, 16, 256
@@ -62,6 +62,7 @@ def load() -> C.CDLL:
     lib.dqlb200_train_host_ext.argtypes = [vp, i32, vp, vp, vp, vp, vp, i32, vp]
     lib.dqlb200_eval_greedy.argtypes = [vp, i32, vp, i64, i64, i32, vp, C.POINTER(K.Trace), i32, vp]
     lib.dqlb200_eval_agents.argtypes = [vp, i32, i64, i64, vp, vp, vp]
+    lib.dqlb200_eval_pairs.argtypes = [vp, C.POINTER(K.Eval2DParams), vp, i32, i64, i64, vp, vp]
     lib.dqlb200_eval_greedy_2d.argtypes = [vp, C.POINTER(K.Eval2DParams), vp, vp, i64, i64, vp, C.POINTER(K.Trace2D), i32, vp]
     lib.dqlb200_bench_table_rmw.argtypes = [vp, vp, i64, i32, i32, i32, vp, vp]
     lib.dqlb200_train_merged.argtypes = [vp, i32, i32, i32, vp]

@@ -35,7 +35,7 @@ EPS_LUT = 2002
 MAX_SETPOINTS = 64              # DQLB200_MAX_SETPOINTS
 MAX_WINDOW = 128
 ENV_STATE_BYTES = 48
-ABI_VERSION = 9
+ABI_VERSION = 10
 
 LIMITS_POSITION = [1.0, 0.64, 0.4096, 0.262144, 0.16777216]   # PKG/mdp.py:45-47
 LIMITS_VELOCITY = [1.0, 0.8, 0.64, 0.512, 0.4096]              # PKG/mdp.py:48-50

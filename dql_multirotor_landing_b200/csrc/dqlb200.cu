@@ -11,7 +11,8 @@
 //                        transfer (R13/R14).  Q_a / count live in shared memory for the whole launch.
 //   env_kernels.cuh      reset_kernel (R1 + R8 for every env), eval_kernel / eval2d_kernel (R15: greedy SimulationMdp
 //                        episodes, one thread per episode, one or two axes), eval_agents_kernel (every agent's greedy policy
-//                        from its live tables, one launch), env_reset_kernel / env_step_kernel (gym surface)
+//                        from its live tables, one launch), eval_pairs_kernel (every x/y agent pair's two-axis landing from
+//                        the live tables, one launch), env_reset_kernel / env_step_kernel (gym surface)
 //   facade_kernels.cuh   float64 single-object TrainingMdp / SimulationMdp / DoubleQLearningAgent calls, division self-test
 //   table_kernels.cuh    transfer (R13), shared-table pack/apply, replica merge, atomic-roof micro-benchmark
 //
@@ -29,6 +30,7 @@
 #include <cstring>
 #include <new>
 #include <string>
+#include <vector>
 #include <dlfcn.h>
 
 
@@ -57,6 +59,11 @@ struct dqlb200_handle {
   void* filter_state;       // accel_mode != 0: [n_total] x 16 B estimator state (dqlb200_bind_filter_state)
   void* dynamics_state;     // dynamics_model != 0: [2][n_total] x 16 B second-order model state (dqlb200_bind_dynamics_state)
   bool kc_default;              // the configuration equals the compile-time defaults: the production instance may run
+  std::vector<int32_t> pop_axis;    // host copy of every population's axis (dqlb200_eval_pairs validates pairs without a device read)
+  std::vector<int32_t> pairs_stage;  // dqlb200_eval_pairs: the caller's pair list, copied here before the (staged) upload
+  int32_t* d_pairs;                 // dqlb200_eval_pairs: the uploaded pair list, grown on demand
+  int d_pairs_cap;
+  cudaEvent_t pairs_read;           // recorded after the launch that reads d_pairs; the next upload waits for it
   size_t smem_bytes;
   // dqlb200_train_host pipelines the populations in chunks over these streams (copy-in / train / copy-out overlap)
   static constexpr int MAX_HOST_CHUNKS = 64;
@@ -192,6 +199,15 @@ int dqlb200_create(const dqlb200_config* cfg, const float* alpha_luts, const dql
   h->merged_exec = h->merged_exec_multi = nullptr;
   h->merged_k = 0;
   h->merged_promote = 0;
+  try {
+    h->pop_axis.assign(cfg->n_populations, 0);
+  } catch (...) {
+    return fail(DQLB200_ERR_STATE, "out of host memory");
+  }
+  for (int p = 0; p < cfg->n_populations; ++p) h->pop_axis[p] = pop_params[p].axis;
+  h->d_pairs = nullptr;
+  h->d_pairs_cap = 0;
+  h->pairs_read = nullptr;
   CUDA_TRY(cudaMalloc(&h->d_cfg, sizeof(dqlb200_config)));
   CUDA_TRY(cudaMemcpy(h->d_cfg, cfg, sizeof(dqlb200_config), cudaMemcpyHostToDevice));
   const size_t lut_bytes = (size_t)cfg->n_alpha_luts * DQLB200_ALPHA_LUT * sizeof(float);
@@ -238,6 +254,8 @@ int dqlb200_destroy(dqlb200_handle* h) {
   cudaFree(h->d_alpha);
   cudaFree(h->d_pop_params);
   cudaFree(h->d_error);
+  cudaFree(h->d_pairs);
+  if (h->pairs_read) cudaEventDestroy(h->pairs_read);
   if (h->chunk_ready) {
     for (int c = 0; c < dqlb200_handle::MAX_HOST_CHUNKS; ++c) {
       cudaStreamDestroy(h->chunk_stream[c]);
@@ -592,6 +610,60 @@ int dqlb200_eval_greedy_2d(dqlb200_handle* h, const dqlb200_eval2d_params* p, co
     dql::eval2d_kernel<true><<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(h->kc, *p, policy_x, policy_y, first_episode, n_episodes,
                                                                                (dqlb200_eval_stats*)stats_out, tr, trace ? trace_steps : 0);
   CUDA_TRY(cudaGetLastError());
+  return DQLB200_OK;
+}
+
+int dqlb200_eval_pairs(dqlb200_handle* h, const dqlb200_eval2d_params* p, const int32_t* pairs_host, int n_pairs, int64_t first_episode,
+                       int64_t episodes_per_pair, void* stats_out, void* stream) {
+  if (!h) return fail(DQLB200_ERR_ARG, "null handle");
+  if (!p || !pairs_host || !stats_out) return fail(DQLB200_ERR_ARG, "params, pairs and stats_out are required");
+  if (n_pairs < 1) return fail(DQLB200_ERR_ARG, "n_pairs must be >= 1");
+  if (p->trajectory < 0 || p->trajectory > 2) return fail(DQLB200_ERR_ARG, "trajectory must be 0 (rectilinear x), 1 (rectilinear x and y) or 2 (eight)");
+  if (p->working_step < -1 || p->working_step >= h->cfg.curriculum_steps)
+    return fail(DQLB200_ERR_ARG, "working_step must be -1 (the lower live step of each pair) or 0 .. curriculum_steps - 1");
+  const int R = h->cfg.replicas_per_population, n_agents = h->cfg.n_populations / R;
+  for (int k = 0; k < n_pairs; ++k) {
+    const int gx = pairs_host[2 * k], gy = pairs_host[2 * k + 1];
+    if (gx < 0 || gx >= n_agents || gy < 0 || gy >= n_agents)
+      return fail(DQLB200_ERR_ARG, "pair " + std::to_string(k) + ": agent index outside 0 .. " + std::to_string(n_agents - 1));
+    if (h->pop_axis[(size_t)gx * R] == 1)
+      return fail(DQLB200_ERR_ARG, "pair " + std::to_string(k) + ": x member " + std::to_string(gx) + " is a y-axis agent");
+  }
+  if (!h->tables || !h->pop_state) return fail(DQLB200_ERR_STATE, "tables / trainer state not bound");
+  if (h->cfg.accel_mode != 0 || h->cfg.dynamics_model != 0)      // refuse rather than silently evaluate on the default model
+    return fail(DQLB200_ERR_ARG, "the two-axis evaluator runs the first-order model with the analytic acceleration only (accel_mode = dynamics_model = 0)");
+  if (episodes_per_pair <= 0) return DQLB200_OK;
+  const long long blocks_per_pair = (episodes_per_pair + 255) / 256;
+  if (blocks_per_pair * n_pairs > 0x7FFFFFFFLL) return fail(DQLB200_ERR_ARG, "episodes_per_pair * n_pairs exceeds one launch's grid");
+  try {
+    h->pairs_stage.assign(pairs_host, pairs_host + (size_t)n_pairs * 2);
+  } catch (...) {
+    return fail(DQLB200_ERR_STATE, "out of host memory");
+  }
+  CUDA_TRY(cudaSetDevice(h->device));
+  cudaStream_t s = (cudaStream_t)stream;
+  if (!h->pairs_read) CUDA_TRY(cudaEventCreateWithFlags(&h->pairs_read, cudaEventDisableTiming));
+  if (n_pairs > h->d_pairs_cap) {
+    CUDA_TRY(cudaEventSynchronize(h->pairs_read));      // the previous launch has read the old list
+    CUDA_TRY(cudaFree(h->d_pairs));
+    h->d_pairs = nullptr;
+    h->d_pairs_cap = 0;
+    CUDA_TRY(cudaMalloc(&h->d_pairs, (size_t)n_pairs * 2 * sizeof(int32_t)));
+    h->d_pairs_cap = n_pairs;
+  }
+  CUDA_TRY(cudaStreamWaitEvent(s, h->pairs_read, 0));      // a launch on another stream may still read the list
+  // from pageable memory the copy is staged before cudaMemcpyAsync returns, so neither pairs_host nor pairs_stage is read later
+  CUDA_TRY(cudaMemcpyAsync(h->d_pairs, h->pairs_stage.data(), (size_t)n_pairs * 2 * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+  const unsigned grid = (unsigned)(blocks_per_pair * n_pairs);
+  const auto* ps = (const dqlb200_population_state*)h->pop_state;
+  if (h->kc_default)
+    dql::eval_pairs_kernel<false><<<grid, 256, 0, s>>>(h->kc, *p, h->d_pop_params, (const uint32_t*)h->tables, ps, h->d_pairs, R,
+                                                      (int)blocks_per_pair, first_episode, episodes_per_pair, (dqlb200_eval_stats*)stats_out);
+  else
+    dql::eval_pairs_kernel<true><<<grid, 256, 0, s>>>(h->kc, *p, h->d_pop_params, (const uint32_t*)h->tables, ps, h->d_pairs, R,
+                                                     (int)blocks_per_pair, first_episode, episodes_per_pair, (dqlb200_eval_stats*)stats_out);
+  CUDA_TRY(cudaGetLastError());
+  CUDA_TRY(cudaEventRecord(h->pairs_read, s));
   return DQLB200_OK;
 }
 

@@ -337,6 +337,77 @@ __device__ __forceinline__ Platform2D platform_2d(const dqlb200_eval2d_params& p
   return m;
 }
 
+// One greedy two-axis episode of the shared-memory LUTs s_pol_x / s_pol_y: the reset draw of episode `ep` under p's key, the
+// hover step, the sub-step loop, both discretisations, the check chain and the optional per-step trace (row `i` of arrays
+// [trace_steps][n_episodes]).  Returns the termination code; `step` = its length.
+template <class KT>
+__device__ __forceinline__ int greedy_episode_2d(const KT& kk, const dqlb200_eval2d_params& p, const dqlb200_cuts& cuts,
+                                                 const uint8_t* s_pol_x, const uint8_t* s_pol_y, unsigned long long ep,
+                                                 const dqlb200_trace2d& trace, int trace_steps, long long i, long long n_episodes,
+                                                 int& step) {
+  const uint4 d = philox4x32_10(make_uint4((uint32_t)ep, 0u, PURPOSE_RESET, p.stream_id), p.seed_lo, p.seed_hi);
+  // PKG/landing_simulation_env.py:327-340: uniform offsets inside the fly zone, absolute clip, random platform phase
+  const float x_init = fadd(-kk.p_max_f, fmul(kk.two_p_max_f, fmul(__uint2float_rn(d.x >> 8), (float)(1.0 / 16777216.0))));
+  const float y_init = fadd(-kk.p_max_f, fmul(kk.two_p_max_f, fmul(__uint2float_rn(d.y >> 8), (float)(1.0 / 16777216.0))));
+  uint32_t phase_x = d.z, phase_y = (p.trajectory == 2) ? d.z : d.w;
+  Platform2D m = platform_2d(p, phase_x, phase_y);
+  Axis bx, by;
+  bx.pos = clipf(fsub(m.xm, x_init), -kk.p_max_f, kk.p_max_f);
+  by.pos = p.y_init_enabled ? clipf(fsub(m.ym, y_init), -kk.p_max_f, kk.p_max_f) : 0.0f;
+  bx.vel = bx.ang = bx.acc = by.vel = by.ang = by.acc = 0.0f;
+  double sp_x = 0.0, sp_y = 0.0;
+  int code = DQLB200_NON_TERMINAL;
+  step = -1;
+  uint32_t sid_x = 0, sid_y = 0;
+  while (code < DQLB200_TERMINAL_SUCCESS) {
+    int ax = 255, ay = 255;
+    if (step >= 0) {          // step == -1: the hover period after the reset (PKG/landing_simulation_env.py:222-224)
+      ax = s_pol_x[sid_x];
+      ay = s_pol_y[sid_y];
+      sp_x = apply_action(kk, sp_x, ax);
+      if (p.y_action_enabled) sp_y = apply_action(kk, sp_y, ay);
+    }
+    for (int k = 0; k < kk.n_sub; ++k) {
+      axis_advance(kk, bx, (float)sp_x, p.g_x);
+      axis_advance(kk, by, (float)sp_y, p.g_y);
+      phase_x += p.dphase_x;
+      phase_y += p.dphase_y;
+    }
+    step += 1;
+    m = platform_2d(p, phase_x, phase_y);
+    Obs ox, oy;
+    ox.rel_p = fsub(m.xm, bx.pos); ox.rel_v = fsub(m.um, bx.vel); ox.rel_a = fsub(m.axm, bx.acc); ox.pitch = bx.ang;
+    oy.rel_p = fsub(m.ym, by.pos); oy.rel_v = fsub(m.vm, by.vel); oy.rel_a = fsub(m.aym, by.acc); oy.pitch = by.ang;
+    const float z = fadd(kk.z_init, fmul(__int2float_rn(step), kk.dz_sim));
+    const bool contact = (z <= kk.z_touch) && (fabsf(ox.rel_p) <= kk.half_platform) && (fabsf(oy.rel_p) <= kk.half_platform);
+    sid_x = (uint32_t)discretise_cuts(cuts, kk.angle_cut, ox).id();
+    sid_y = (uint32_t)discretise_cuts(cuts, kk.angle_cut, oy).id();
+    if (step == 0) continue;          // the reset only observes (no check, PKG/landing_simulation_env.py:236-243)
+    if (contact) code = DQLB200_TERMINAL_CONTACT;
+    else if (!(ox.rel_p >= kk.fz_lo) || (ox.rel_p >= kk.fz_hi)) code = DQLB200_TERMINAL_FLYZONE_X;
+    else if (!(oy.rel_p >= kk.fz_lo) || (oy.rel_p >= kk.fz_hi)) code = DQLB200_TERMINAL_FLYZONE_Y;
+    else if (!(z >= kk.z_min_cut)) code = DQLB200_TERMINAL_MINIMUM_ALTITUDE;
+    else if (z >= kk.z_max_cut) code = DQLB200_TERMINAL_FLYZONE_Z;
+    else if (step >= kk.timeout_steps) code = DQLB200_TERMINAL_TIMEOUT;
+    if (step <= trace_steps) {
+      const size_t ti = (size_t)(step - 1) * (size_t)n_episodes + (size_t)i;
+      if (trace.obs) {
+        float* po = trace.obs + ti * 9;
+        po[0] = ox.rel_p; po[1] = ox.rel_v; po[2] = ox.rel_a; po[3] = ox.pitch; po[4] = z;
+        po[5] = oy.rel_p; po[6] = oy.rel_v; po[7] = oy.rel_a; po[8] = oy.pitch;
+      }
+      if (trace.action_x) trace.action_x[ti] = (uint8_t)ax;
+      if (trace.action_y) trace.action_y[ti] = (uint8_t)ay;
+      if (trace.code) trace.code[ti] = (uint8_t)code;
+      if (trace.done) trace.done[ti] = (uint8_t)(code >= DQLB200_TERMINAL_SUCCESS);
+      if (trace.contact) trace.contact[ti] = (uint8_t)contact;
+      if (trace.state_x) trace.state_x[ti] = (uint16_t)sid_x;
+      if (trace.state_y) trace.state_y[ti] = (uint16_t)sid_y;
+    }
+  }
+  return code;
+}
+
 template <bool GENERIC>
 __global__ void __launch_bounds__(256) eval2d_kernel(const __grid_constant__ KC kc, const __grid_constant__ dqlb200_eval2d_params p,
                                                      const uint8_t* __restrict__ policy_x, const uint8_t* __restrict__ policy_y,
@@ -355,66 +426,9 @@ __global__ void __launch_bounds__(256) eval2d_kernel(const __grid_constant__ KC 
   __syncthreads();
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n_episodes) {
-    const unsigned long long ep = (unsigned long long)(first_episode + i);
-    const uint4 d = philox4x32_10(make_uint4((uint32_t)ep, 0u, PURPOSE_RESET, p.stream_id), p.seed_lo, p.seed_hi);
-    // PKG/landing_simulation_env.py:327-340: uniform offsets inside the fly zone, absolute clip, random platform phase
-    const float x_init = fadd(-kk.p_max_f, fmul(kk.two_p_max_f, fmul(__uint2float_rn(d.x >> 8), (float)(1.0 / 16777216.0))));
-    const float y_init = fadd(-kk.p_max_f, fmul(kk.two_p_max_f, fmul(__uint2float_rn(d.y >> 8), (float)(1.0 / 16777216.0))));
-    uint32_t phase_x = d.z, phase_y = (p.trajectory == 2) ? d.z : d.w;
-    Platform2D m = platform_2d(p, phase_x, phase_y);
-    Axis bx, by;
-    bx.pos = clipf(fsub(m.xm, x_init), -kk.p_max_f, kk.p_max_f);
-    by.pos = p.y_init_enabled ? clipf(fsub(m.ym, y_init), -kk.p_max_f, kk.p_max_f) : 0.0f;
-    bx.vel = bx.ang = bx.acc = by.vel = by.ang = by.acc = 0.0f;
-    double sp_x = 0.0, sp_y = 0.0;
-    int code = DQLB200_NON_TERMINAL, step = -1;
-    uint32_t sid_x = 0, sid_y = 0;
-    while (code < DQLB200_TERMINAL_SUCCESS) {
-      int ax = 255, ay = 255;
-      if (step >= 0) {          // step == -1: the hover period after the reset (PKG/landing_simulation_env.py:222-224)
-        ax = s_pol_x[sid_x];
-        ay = s_pol_y[sid_y];
-        sp_x = apply_action(kk, sp_x, ax);
-        if (p.y_action_enabled) sp_y = apply_action(kk, sp_y, ay);
-      }
-      for (int k = 0; k < kk.n_sub; ++k) {
-        axis_advance(kk, bx, (float)sp_x, p.g_x);
-        axis_advance(kk, by, (float)sp_y, p.g_y);
-        phase_x += p.dphase_x;
-        phase_y += p.dphase_y;
-      }
-      step += 1;
-      m = platform_2d(p, phase_x, phase_y);
-      Obs ox, oy;
-      ox.rel_p = fsub(m.xm, bx.pos); ox.rel_v = fsub(m.um, bx.vel); ox.rel_a = fsub(m.axm, bx.acc); ox.pitch = bx.ang;
-      oy.rel_p = fsub(m.ym, by.pos); oy.rel_v = fsub(m.vm, by.vel); oy.rel_a = fsub(m.aym, by.acc); oy.pitch = by.ang;
-      const float z = fadd(kk.z_init, fmul(__int2float_rn(step), kk.dz_sim));
-      const bool contact = (z <= kk.z_touch) && (fabsf(ox.rel_p) <= kk.half_platform) && (fabsf(oy.rel_p) <= kk.half_platform);
-      sid_x = (uint32_t)discretise_cuts(cuts, kk.angle_cut, ox).id();
-      sid_y = (uint32_t)discretise_cuts(cuts, kk.angle_cut, oy).id();
-      if (step == 0) continue;          // the reset only observes (no check, PKG/landing_simulation_env.py:236-243)
-      if (contact) code = DQLB200_TERMINAL_CONTACT;
-      else if (!(ox.rel_p >= kk.fz_lo) || (ox.rel_p >= kk.fz_hi)) code = DQLB200_TERMINAL_FLYZONE_X;
-      else if (!(oy.rel_p >= kk.fz_lo) || (oy.rel_p >= kk.fz_hi)) code = DQLB200_TERMINAL_FLYZONE_Y;
-      else if (!(z >= kk.z_min_cut)) code = DQLB200_TERMINAL_MINIMUM_ALTITUDE;
-      else if (z >= kk.z_max_cut) code = DQLB200_TERMINAL_FLYZONE_Z;
-      else if (step >= kk.timeout_steps) code = DQLB200_TERMINAL_TIMEOUT;
-      if (step <= trace_steps) {
-        const size_t ti = (size_t)(step - 1) * (size_t)n_episodes + (size_t)i;
-        if (trace.obs) {
-          float* po = trace.obs + ti * 9;
-          po[0] = ox.rel_p; po[1] = ox.rel_v; po[2] = ox.rel_a; po[3] = ox.pitch; po[4] = z;
-          po[5] = oy.rel_p; po[6] = oy.rel_v; po[7] = oy.rel_a; po[8] = oy.pitch;
-        }
-        if (trace.action_x) trace.action_x[ti] = (uint8_t)ax;
-        if (trace.action_y) trace.action_y[ti] = (uint8_t)ay;
-        if (trace.code) trace.code[ti] = (uint8_t)code;
-        if (trace.done) trace.done[ti] = (uint8_t)(code >= DQLB200_TERMINAL_SUCCESS);
-        if (trace.contact) trace.contact[ti] = (uint8_t)contact;
-        if (trace.state_x) trace.state_x[ti] = (uint16_t)sid_x;
-        if (trace.state_y) trace.state_y[ti] = (uint16_t)sid_y;
-      }
-    }
+    int step;
+    const int code = greedy_episode_2d(kk, p, cuts, s_pol_x, s_pol_y, (unsigned long long)(first_episode + i), trace, trace_steps, i,
+                                       n_episodes, step);
     atomicAdd(&s_hist[code], 1u);
     atomicAdd(&s_steps, (unsigned int)step);
     atomicAdd(&s_eps, 1u);
@@ -424,6 +438,76 @@ __global__ void __launch_bounds__(256) eval2d_kernel(const __grid_constant__ KC 
   if (threadIdx.x == 0) {
     atomicAdd((unsigned long long*)&stats->steps, (unsigned long long)s_steps);
     atomicAdd((unsigned long long*)&stats->episodes, (unsigned long long)s_eps);
+  }
+}
+
+// Every (x agent, y agent) pair's two-axis greedy landing in one launch: blocks_per_pair blocks of 256 episodes per pair on a
+// flat 1-D grid (pair = blockIdx.x / blocks_per_pair).  Pair k = (gx, gy) = pairs[2k], pairs[2k + 1]; agent g reads replica
+// g * replicas.  Each block builds both LUTs in shared memory from the live tables: x from gx's float32 first-max; y from gy's
+// own float32 first-max when gy is a y-axis agent (population axis 1), else the mirror image of gy's x policy
+// (lut_y[s] = {1,0,2}[lut(rest * 7 + 6 - theta)], rest, theta = divmod(s, 7): engine.mirrored_policy).  States at and above
+// curriculum_steps * 189 act 0 on both axes.  Platform, gravity signs, y options and Philox key come from p for every pair, so
+// episode i of every pair starts from the same draw: episode first_episode + i of eval2d_kernel under the two LUTs.  p.working_step
+// < 0: the lower of the two members' live working steps.  Reads tables and trainer state, writes only stats.
+template <bool GENERIC>
+__global__ void __launch_bounds__(256) eval_pairs_kernel(const __grid_constant__ KC kc, const __grid_constant__ dqlb200_eval2d_params p,
+                                                         const dqlb200_population_params* pop_params, const uint32_t* __restrict__ tables,
+                                                         const dqlb200_population_state* __restrict__ pop_state,
+                                                         const int32_t* __restrict__ pairs, int replicas, int blocks_per_pair,
+                                                         long long first_episode, long long episodes_per_pair, dqlb200_eval_stats* stats) {
+  const auto& kk = ConstsOf<GENERIC>::get(kc);
+  constexpr int N_STATES = DQLB200_MAX_CURRICULUM * DQLB200_STATES_PER_LEVEL;
+  __shared__ uint8_t s_pol_x[N_STATES], s_pol_y[N_STATES];
+  __shared__ dqlb200_cuts cuts;
+  __shared__ unsigned int s_hist[9], s_steps, s_eps;
+  const int pair = (int)(blockIdx.x / (unsigned)blocks_per_pair);
+  const int block_in_pair = (int)(blockIdx.x - (unsigned)pair * (unsigned)blocks_per_pair);
+  const int pop_x = pairs[2 * pair] * replicas, pop_y = pairs[2 * pair + 1] * replicas;
+  const float* qax = reinterpret_cast<const float*>(tables + (size_t)pop_x * 3 * DQLB200_MAX_CELLS);
+  const float* qbx = qax + DQLB200_MAX_CELLS;
+  const float* qay = reinterpret_cast<const float*>(tables + (size_t)pop_y * 3 * DQLB200_MAX_CELLS);
+  const float* qby = qay + DQLB200_MAX_CELLS;
+  const bool y_own = pop_params[pop_y].axis == 1;
+  const int live_states = kc.curriculum_steps * DQLB200_STATES_PER_LEVEL;
+  for (int s = threadIdx.x; s < N_STATES; s += blockDim.x) {
+    uint8_t ax = 0, ay = 0;
+    if (s < live_states) {
+      ax = greedy_action_f32(qax, qbx, s);
+      if (y_own) {
+        ay = greedy_action_f32(qay, qby, s);
+      } else {
+        const int rest = s / 7, theta = s - rest * 7;
+        const uint8_t a = greedy_action_f32(qay, qby, rest * 7 + 6 - theta);
+        ay = a == 2 ? (uint8_t)2 : (uint8_t)(1 - a);      // {1, 0, 2}[a]: increase and decrease swap
+      }
+    }
+    s_pol_x[s] = ax;
+    s_pol_y[s] = ay;
+  }
+  if (threadIdx.x == 0) {
+    int w = p.working_step;
+    if (w < 0) w = min(max(min(pop_state[pop_x].working_step, pop_state[pop_y].working_step), 0), kc.curriculum_steps - 1);
+    cuts = kc.cuts[w];
+    s_steps = s_eps = 0u;
+  }
+  if (threadIdx.x < 9) s_hist[threadIdx.x] = 0u;
+  __syncthreads();
+  const long long i = (long long)block_in_pair * blockDim.x + threadIdx.x;
+  if (i < episodes_per_pair) {
+    int step;
+    const dqlb200_trace2d no_trace = {};
+    const int code = greedy_episode_2d(kk, p, cuts, s_pol_x, s_pol_y, (unsigned long long)(first_episode + i), no_trace, 0, i,
+                                       episodes_per_pair, step);
+    atomicAdd(&s_hist[code], 1u);
+    atomicAdd(&s_steps, (unsigned int)step);
+    atomicAdd(&s_eps, 1u);
+  }
+  __syncthreads();
+  dqlb200_eval_stats* st = stats + pair;
+  if (threadIdx.x < 9 && s_hist[threadIdx.x]) atomicAdd((unsigned long long*)&st->termination_hist[threadIdx.x], (unsigned long long)s_hist[threadIdx.x]);
+  if (threadIdx.x == 0) {
+    atomicAdd((unsigned long long*)&st->steps, (unsigned long long)s_steps);
+    atomicAdd((unsigned long long*)&st->episodes, (unsigned long long)s_eps);
   }
 }
 

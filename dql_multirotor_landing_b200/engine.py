@@ -355,6 +355,38 @@ class Engine:
         torch.cuda.synchronize(dev)
         return _eval_result(K.EvalStats.from_buffer_copy(stats.cpu().numpy().tobytes()), out)
 
+    def eval_pairs(self, episodes_per_pair: int, pairs: Sequence[Sequence[int]], *, two_axis: Optional[K.TwoAxisParameters] = None,
+                   seed: int = 42, stream_id: int = 0, first_episode: int = 0, working_step: Optional[int] = None) -> dict:
+        """Greedy two-axis SimulationMdp episodes of every (x agent, y agent) pair, both LUTs built on the device from the live
+        float32 tables (dqlb200_eval_pairs): one launch, one copy back, one synchronisation.  pairs: (gx, gy) agent indices
+        (agent g = replica group g, population g * R); gx must be an x agent.  gy a y agent flies y with its own policy, gy an
+        x agent with the mirror image of its policy (mirrored_policy).  working_step None = the lower of the two members' live
+        working steps.  Pair k's episodes are those of eval_greedy_2d(<lut_x>, <lut_y>, episodes_per_pair, two_axis=...,
+        seed=..., stream_id=..., first_episode=..., working_step=...), the same initial conditions for every pair.  Returns
+        NumPy arrays over the pairs: pairs [K, 2], episodes [K], steps [K], termination_hist [K, 9], success_rate [K] (goal or
+        contact)."""
+        pr = np.asarray(pairs, dtype=np.int64)
+        if pr.size == 0:
+            pr = pr.reshape(0, 2)
+        if pr.ndim != 2 or pr.shape[1] != 2:
+            raise ValueError("pairs must be a sequence of (gx, gy) agent indices")
+        if pr.size and (pr.min() < np.iinfo(np.int32).min or pr.max() > np.iinfo(np.int32).max):
+            raise ValueError("agent index out of range")
+        host_pairs = np.ascontiguousarray(pr, dtype=np.int32)
+        n = len(host_pairs)
+        w = -1 if working_step is None else int(working_step)
+        prm = K.eval2d_params(two_axis or K.TwoAxisParameters(), self.dp, self.mp.f_ag, seed, stream_id, w)
+        stats_bytes = n * C.sizeof(K.EvalStats)
+        buf = torch.zeros(max(stats_bytes, 1), dtype=torch.uint8, device=self.device)
+        _ffi.check(self.lib.dqlb200_eval_pairs(self.handle, C.byref(prm), host_pairs.ctypes.data, n, int(first_episode),
+                                               int(episodes_per_pair), buf.data_ptr(), self._stream()))
+        host = buf.cpu().numpy()          # synchronises the stream
+        st = host[:stats_bytes].view(np.uint64).reshape(n, 11).astype(np.int64)
+        res = dict(pairs=pr, episodes=st[:, 0], steps=st[:, 1], termination_hist=st[:, 2:])
+        hist = res["termination_hist"]            # codes 2 (goal) and 3 (contact), as eval_agents
+        res["success_rate"] = (hist[:, 2] + hist[:, 3]) / np.maximum(res["episodes"], 1)
+        return res
+
 
 def eight_axis_platforms(r: float = 3.0, v: float = 0.8):
     """(r_mp, v_mp) of the x and the y agent for decoupled training under the reference's "eight" platform trajectory

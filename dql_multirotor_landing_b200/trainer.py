@@ -47,6 +47,7 @@ def replica_shape(num_envs: int, merge_every: int = 1) -> int:
 class Trainer:
     _eval_every: Optional[int] = None       # greedy evaluation of every agent after each `eval_every`-th chunk (None: off)
     _eval_episodes: int = 1024
+    _eval_two_axis: Optional[K.TwoAxisParameters] = None      # also the two-axis landing (x policy on x, its mirror on y)
 
     def __init__(
         self,
@@ -84,6 +85,7 @@ class Trainer:
         direction: str = "x",
         eval_every: Optional[int] = None,
         eval_episodes: int = 1024,
+        eval_two_axis: Optional[K.TwoAxisParameters] = None,
     ) -> None:
         np.random.seed(seed)                                        # PKG/trainer.py:45
         if not double_q_learning_agent:
@@ -128,6 +130,14 @@ class Trainer:
             if eval_every < 1 or eval_episodes < 1:
                 raise ValueError("eval_every and eval_episodes must be >= 1")
             self._eval_every, self._eval_episodes = eval_every, eval_episodes
+        if eval_two_axis is not None:       # likewise stored only when set
+            if eval_every is None:
+                raise ValueError("eval_two_axis needs eval_every")
+            if direction != "x":
+                raise ValueError("eval_two_axis flies the x agent on both axes: it needs direction='x'")
+            if self._dynamics.accel_mode != "exact" or self._dynamics.dynamics_model != "first_order":
+                raise ValueError("eval_two_axis runs the first-order model with the exact acceleration only")
+            self._eval_two_axis = eval_two_axis
         self._engine = None
         self.history = []             # one dict per chunk (population 0)
 
@@ -262,6 +272,11 @@ class Trainer:
                 rates = eng.eval_agents(self._eval_episodes)["success_rate"]      # greedy policies at the live working steps
                 info["Greedy success rate"] = float(rates[0])
                 entry["Greedy success rates"] = [float(r) for r in rates]
+                if self._eval_two_axis is not None:      # every agent on both axes: its policy on x, the mirror image on y
+                    rates2 = eng.eval_pairs(self._eval_episodes, [(g, g) for g in range(len(rates))],
+                                            two_axis=self._eval_two_axis)["success_rate"]
+                    info["Greedy two-axis success rate"] = float(rates2[0])
+                    entry["Greedy two-axis success rates"] = [float(r) for r in rates2]
             self.history.append(dict(info, working_step=self._working_curriculum_step, **entry))
             if len(self.history) > 2048:          # bounded: the history is pickled with every checkpoint
                 del self.history[:1024]
@@ -295,6 +310,8 @@ class Trainer:
             writer.add_scalar("Episode/Mean reward", info["Mean reward"], step)
             if "Greedy success rate" in info:
                 writer.add_scalar("Episode/Greedy Success Rate", info["Greedy success rate"], step)
+            if "Greedy two-axis success rate" in info:
+                writer.add_scalar("Episode/Greedy Two-Axis Success Rate", info["Greedy two-axis success rate"], step)
             writer.add_text("Episode/Termination Condition", info["Termination condition"], step)
             writer.close()
         if clean:

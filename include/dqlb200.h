@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define DQLB200_ABI_VERSION 9
+#define DQLB200_ABI_VERSION 10
 #define DQLB200_MAX_CURRICULUM 5
 #define DQLB200_STATES_PER_LEVEL 189          /* 3*3*3*7      (PKG/double_q_learning.py:38-40) */
 #define DQLB200_CELLS_PER_LEVEL 567           /* 189 * 3 actions */
@@ -384,6 +384,37 @@ int dqlb200_agent_update(dqlb200_handle* h, const uint16_t* states, const uint8_
 int dqlb200_eval_greedy_2d(dqlb200_handle* h, const dqlb200_eval2d_params* p, const uint8_t* policy_x,
                            const uint8_t* policy_y, int64_t first_episode, int64_t n_episodes, void* stats_out,
                            const dqlb200_trace2d* trace, int trace_steps, void* stream);
+
+/* dqlb200_eval_greedy_2d for MANY (x agent, y agent) pairs at once, each pair's two LUTs built on the device from the bound
+ * float32 tables: one launch, no host round trip per pair.
+ *   pairs_host   : host int32 [n_pairs][2] = (gx, gy), agent indices 0 .. n_populations / R - 1 (R = replicas_per_population;
+ *                  agent g is the replica group g*R .. g*R+R-1, read through replica g*R: its tables, its axis, its trainer
+ *                  state).  The list is validated on the host, copied into a library-owned host buffer and from there to a
+ *                  library-owned device buffer on `stream`: pairs_host (pageable or pinned) is never read after the call
+ *                  returns, so the caller may reuse it at once.  An agent may appear in any number of pairs.
+ *   x LUT        : for every state s < curriculum_steps * 189 the FIRST maximum over a of float32 (Q_a[s,a] + Q_b[s,a]) * 0.5f
+ *                  of agent gx, each operation rounded to nearest (the policy dqlb200_eval_agents evaluates); gx must be an
+ *                  x-axis agent (dqlb200_population_params.axis 0).
+ *   y LUT        : gy a y-axis agent (axis 1): its own float32 first-max LUT.  gy an x-axis agent: the mirror image of its
+ *                  float32 LUT, lut_y[s] = {1,0,2}[lut(rest*7 + 6 - theta)] with rest, theta = divmod(s, 7) (the rule of
+ *                  engine.mirrored_policy: the state with the mirrored angle index, increase and decrease swapped), so one
+ *                  agent trained on x flies both axes as the reference's scripts/simulation.py does.
+ *                  States at and above curriculum_steps * 189 act 0 on both axes.
+ *   p            : platform, gravity signs, y options and the Philox key (seed, stream_id) of the whole launch: every pair
+ *                  sees the same episodes' initial conditions, so differences between pairs are differences of policy.
+ *                  p->working_step >= 0 evaluates every pair under the cut table of that step; -1 (allowed here only) takes
+ *                  the lower of the two members' live dqlb200_population_state.working_step, read on the device and clamped
+ *                  to 0 .. curriculum_steps - 1.
+ *   episodes     : episode i of pair k is, one for one, episode first_episode + i of dqlb200_eval_greedy_2d(p, lut_x, lut_y)
+ *                  with that pair's LUTs and working step.
+ *   stats_out    : device dqlb200_eval_stats[n_pairs], accumulated (the caller zeroes), exact integer counts.
+ * Nothing bound is written: env state, tables and trainer state are only read.
+ * Refused (DQLB200_ERR_ARG): a NULL handle, p, pairs_host or stats_out; n_pairs < 1; an agent index out of range; an x member
+ * that is a y-axis agent; trajectory outside 0..2; working_step outside -1 .. curriculum_steps - 1; accel_mode != 0 or
+ * dynamics_model != 0 (as dqlb200_eval_greedy_2d); more than 0x7FFFFFFF blocks.  Tables or trainer state not bound:
+ * DQLB200_ERR_STATE.  episodes_per_pair <= 0 does nothing. */
+int dqlb200_eval_pairs(dqlb200_handle* h, const dqlb200_eval2d_params* p, const int32_t* pairs_host, int n_pairs,
+                       int64_t first_episode, int64_t episodes_per_pair, void* stats_out, void* stream);
 
 /* Replaces: DoubleQLearningAgent.transfer_learning (PKG/double_q_learning.py:77-89) on the bound
  * tables of every population. */
