@@ -35,7 +35,7 @@ EPS_LUT = 2002
 MAX_SETPOINTS = 64              # DQLB200_MAX_SETPOINTS
 MAX_WINDOW = 128
 ENV_STATE_BYTES = 48
-ABI_VERSION = 10
+ABI_VERSION = 11
 
 LIMITS_POSITION = [1.0, 0.64, 0.4096, 0.262144, 0.16777216]   # PKG/mdp.py:45-47
 LIMITS_VELOCITY = [1.0, 0.8, 0.64, 0.512, 0.4096]              # PKG/mdp.py:48-50
@@ -148,6 +148,12 @@ class Trace(C.Structure):
 
 class EvalStats(C.Structure):
     _fields_ = [("episodes", C.c_uint64), ("steps", C.c_uint64), ("termination_hist", C.c_uint64 * 9)]
+
+
+class Platform(C.Structure):
+    """dqlb200_platform (include/dqlb200.h): one platform motion of dqlb200_eval_agents_platforms, the fields of
+    PopulationParams with the same names (platform_constants)."""
+    _fields_ = [("dphase", C.c_uint32), ("r", C.c_float), ("rw", C.c_float), ("rw2", C.c_float)]
 
 
 class Eval2DParams(C.Structure):
@@ -470,6 +476,22 @@ def platform_constants(r_mp: float, v_mp: float, f_ag: float, n_sub: int):
     w = v_mp / r_mp
     dphase = int(round(w * h / (2.0 * math.pi) * 2.0 ** 32)) & 0xFFFFFFFF
     return dphase, np.float32(r_mp), np.float32(r_mp * w), np.float32(r_mp * w * w)
+
+
+def platform_motions(platforms) -> np.ndarray:
+    """A list of platform motions (r_mp, v_mp) as float64 [C, 2]; ValueError for an empty list, a wrong shape, a non-finite value,
+    r_mp <= 0 or v_mp < 0."""
+    try:
+        pl = np.asarray(platforms, dtype=np.float64)
+    except (TypeError, ValueError) as e:
+        raise ValueError(f"platforms must be a sequence of (r_mp, v_mp) pairs: {e}") from None
+    if pl.ndim != 2 or pl.shape[1] != 2 or len(pl) < 1:
+        raise ValueError(f"platforms must be a non-empty sequence of (r_mp, v_mp) pairs, got shape {pl.shape}")
+    if not np.isfinite(pl).all():
+        raise ValueError("platforms: r_mp and v_mp must be finite")
+    if not (pl[:, 0] > 0).all() or not (pl[:, 1] >= 0).all():
+        raise ValueError("platforms: r_mp must be > 0 and v_mp >= 0")
+    return pl
 
 
 def build_config(n_populations: int, envs_per_population: int, threads_per_block: int = 256,

@@ -11,7 +11,8 @@
 //                        transfer (R13/R14).  Q_a / count live in shared memory for the whole launch.
 //   env_kernels.cuh      reset_kernel (R1 + R8 for every env), eval_kernel / eval2d_kernel (R15: greedy SimulationMdp
 //                        episodes, one thread per episode, one or two axes), eval_agents_kernel (every agent's greedy policy
-//                        from its live tables, one launch), eval_pairs_kernel (every x/y agent pair's two-axis landing from
+//                        from its live tables, one launch, under its own platform or a list of platform motions),
+//                        eval_pairs_kernel (every x/y agent pair's two-axis landing from
 //                        the live tables, one launch), env_reset_kernel / env_step_kernel (gym surface)
 //   facade_kernels.cuh   float64 single-object TrainingMdp / SimulationMdp / DoubleQLearningAgent calls, division self-test
 //   table_kernels.cuh    transfer (R13), shared-table pack/apply, replica merge, atomic-roof micro-benchmark
@@ -64,6 +65,10 @@ struct dqlb200_handle {
   int32_t* d_pairs;                 // dqlb200_eval_pairs: the uploaded pair list, grown on demand
   int d_pairs_cap;
   cudaEvent_t pairs_read;           // recorded after the launch that reads d_pairs; the next upload waits for it
+  std::vector<dqlb200_platform> platforms_stage;   // dqlb200_eval_agents_platforms: the caller's list, staged as pairs_stage
+  dqlb200_platform* d_platforms;                   // the uploaded list, grown on demand
+  int d_platforms_cap;
+  cudaEvent_t platforms_read;                      // recorded after the launch that reads d_platforms
   size_t smem_bytes;
   // dqlb200_train_host pipelines the populations in chunks over these streams (copy-in / train / copy-out overlap)
   static constexpr int MAX_HOST_CHUNKS = 64;
@@ -96,6 +101,7 @@ int dqlb200_abi_version(void) { return DQLB200_ABI_VERSION; }
 size_t dqlb200_config_bytes(void) { return sizeof(dqlb200_config); }
 size_t dqlb200_population_state_bytes(void) { return sizeof(dqlb200_population_state); }
 size_t dqlb200_eval2d_params_bytes(void) { return sizeof(dqlb200_eval2d_params); }
+size_t dqlb200_platform_bytes(void) { return sizeof(dqlb200_platform); }
 size_t dqlb200_env_state_bytes(int n_populations, int envs_per_population) {
   if (n_populations < 0 || envs_per_population < 0) return 0;
   return (size_t)n_populations * (((size_t)envs_per_population + 31) / 32) * dql::ENV_TILE_BYTES;
@@ -208,6 +214,9 @@ int dqlb200_create(const dqlb200_config* cfg, const float* alpha_luts, const dql
   h->d_pairs = nullptr;
   h->d_pairs_cap = 0;
   h->pairs_read = nullptr;
+  h->d_platforms = nullptr;
+  h->d_platforms_cap = 0;
+  h->platforms_read = nullptr;
   CUDA_TRY(cudaMalloc(&h->d_cfg, sizeof(dqlb200_config)));
   CUDA_TRY(cudaMemcpy(h->d_cfg, cfg, sizeof(dqlb200_config), cudaMemcpyHostToDevice));
   const size_t lut_bytes = (size_t)cfg->n_alpha_luts * DQLB200_ALPHA_LUT * sizeof(float);
@@ -256,6 +265,8 @@ int dqlb200_destroy(dqlb200_handle* h) {
   cudaFree(h->d_error);
   cudaFree(h->d_pairs);
   if (h->pairs_read) cudaEventDestroy(h->pairs_read);
+  cudaFree(h->d_platforms);
+  if (h->platforms_read) cudaEventDestroy(h->platforms_read);
   if (h->chunk_ready) {
     for (int c = 0; c < dqlb200_handle::MAX_HOST_CHUNKS; ++c) {
       cudaStreamDestroy(h->chunk_stream[c]);
@@ -507,6 +518,34 @@ int dqlb200_eval_greedy(dqlb200_handle* h, int population, const uint8_t* policy
   return DQLB200_OK;
 }
 
+// ceil(episodes_per_agent / 256) blocks per cell x n_agents x n_platforms cells fit one launch's 1-D grid (episodes_per_agent >= 1;
+// n_agents and n_platforms are below 2^31, so their product does not overflow)
+static bool eval_agents_grid_fits(const dqlb200_handle* h, int64_t episodes_per_agent, int n_platforms) {
+  const long long cells = (long long)(h->cfg.n_populations / h->cfg.replicas_per_population) * n_platforms;
+  return (episodes_per_agent - 1) / 256 + 1 <= 0x7FFFFFFFLL / cells;
+}
+
+// One eval_agents_kernel launch over n_agents x n_platforms cells (d_platforms nullptr: each agent's own platform, n_platforms 1).
+// The caller has checked every argument.
+static int launch_eval_agents(dqlb200_handle* h, int working_step, int64_t first_episode, int64_t episodes_per_agent,
+                              const dqlb200_platform* d_platforms, int n_platforms, void* stats_out, uint8_t* policy_out, cudaStream_t s) {
+  const long long blocks_per_agent = (episodes_per_agent - 1) / 256 + 1;
+  const int R = h->cfg.replicas_per_population, n_agents = h->cfg.n_populations / R;
+  CUDA_TRY(cudaSetDevice(h->device));
+  const unsigned grid = (unsigned)(blocks_per_agent * n_agents * n_platforms);
+  const auto* ps = (const dqlb200_population_state*)h->pop_state;
+  if (h->kc_default)
+    dql::eval_agents_kernel<false><<<grid, 256, 0, s>>>(h->kc, h->d_pop_params, (const uint32_t*)h->tables, ps, R, (int)blocks_per_agent,
+                                                       first_episode, episodes_per_agent, working_step, d_platforms, n_platforms,
+                                                       (dqlb200_eval_stats*)stats_out, policy_out);
+  else
+    dql::eval_agents_kernel<true><<<grid, 256, 0, s>>>(h->kc, h->d_pop_params, (const uint32_t*)h->tables, ps, R, (int)blocks_per_agent,
+                                                      first_episode, episodes_per_agent, working_step, d_platforms, n_platforms,
+                                                      (dqlb200_eval_stats*)stats_out, policy_out);
+  CUDA_TRY(cudaGetLastError());
+  return DQLB200_OK;
+}
+
 int dqlb200_eval_agents(dqlb200_handle* h, int working_step, int64_t first_episode, int64_t episodes_per_agent, void* stats_out,
                         uint8_t* policy_out, void* stream) {
   if (!h) return fail(DQLB200_ERR_ARG, "null handle");
@@ -516,20 +555,51 @@ int dqlb200_eval_agents(dqlb200_handle* h, int working_step, int64_t first_episo
   if (!h->tables || !h->pop_state) return fail(DQLB200_ERR_STATE, "tables / trainer state not bound");
   DQL_NEED_FILTER(h);
   if (episodes_per_agent <= 0) return DQLB200_OK;
-  const long long blocks_per_agent = (episodes_per_agent + 255) / 256;
-  const int R = h->cfg.replicas_per_population, n_agents = h->cfg.n_populations / R;
-  if (blocks_per_agent * n_agents > 0x7FFFFFFFLL) return fail(DQLB200_ERR_ARG, "episodes_per_agent * n_agents exceeds one launch's grid");
+  if (!eval_agents_grid_fits(h, episodes_per_agent, 1)) return fail(DQLB200_ERR_ARG, "episodes_per_agent * n_agents exceeds one launch's grid");
+  return launch_eval_agents(h, working_step, first_episode, episodes_per_agent, nullptr, 1, stats_out, policy_out, (cudaStream_t)stream);
+}
+
+int dqlb200_eval_agents_platforms(dqlb200_handle* h, int working_step, int64_t first_episode, int64_t episodes_per_agent,
+                                  const dqlb200_platform* platforms_host, int n_platforms, void* stats_out, void* stream) {
+  if (!h) return fail(DQLB200_ERR_ARG, "null handle");
+  if (!platforms_host || !stats_out) return fail(DQLB200_ERR_ARG, "platforms_host and stats_out are required");
+  if (n_platforms < 1) return fail(DQLB200_ERR_ARG, "n_platforms must be >= 1");
+  for (int c = 0; c < n_platforms; ++c) {
+    const dqlb200_platform& pl = platforms_host[c];
+    if (!std::isfinite(pl.r) || !(pl.r > 0.0f))
+      return fail(DQLB200_ERR_ARG, "platform " + std::to_string(c) + ": r must be finite and > 0");
+    if (!std::isfinite(pl.rw) || !std::isfinite(pl.rw2) || !(pl.rw >= 0.0f) || !(pl.rw2 >= 0.0f))
+      return fail(DQLB200_ERR_ARG, "platform " + std::to_string(c) + ": rw and rw2 must be finite and >= 0");
+  }
+  if (working_step < -1 || working_step >= h->cfg.curriculum_steps)
+    return fail(DQLB200_ERR_ARG, "working_step must be -1 (each agent's live step) or 0 .. curriculum_steps - 1");
+  if (!h->tables || !h->pop_state) return fail(DQLB200_ERR_STATE, "tables / trainer state not bound");
+  DQL_NEED_FILTER(h);
+  if (episodes_per_agent <= 0) return DQLB200_OK;
+  if (!eval_agents_grid_fits(h, episodes_per_agent, n_platforms))
+    return fail(DQLB200_ERR_ARG, "episodes_per_agent * n_agents * n_platforms exceeds one launch's grid");
+  try {
+    h->platforms_stage.assign(platforms_host, platforms_host + n_platforms);
+  } catch (...) {
+    return fail(DQLB200_ERR_STATE, "out of host memory");
+  }
   CUDA_TRY(cudaSetDevice(h->device));
-  const unsigned grid = (unsigned)(blocks_per_agent * n_agents);
   cudaStream_t s = (cudaStream_t)stream;
-  const auto* ps = (const dqlb200_population_state*)h->pop_state;
-  if (h->kc_default)
-    dql::eval_agents_kernel<false><<<grid, 256, 0, s>>>(h->kc, h->d_pop_params, (const uint32_t*)h->tables, ps, R, (int)blocks_per_agent,
-                                                       first_episode, episodes_per_agent, working_step, (dqlb200_eval_stats*)stats_out, policy_out);
-  else
-    dql::eval_agents_kernel<true><<<grid, 256, 0, s>>>(h->kc, h->d_pop_params, (const uint32_t*)h->tables, ps, R, (int)blocks_per_agent,
-                                                      first_episode, episodes_per_agent, working_step, (dqlb200_eval_stats*)stats_out, policy_out);
-  CUDA_TRY(cudaGetLastError());
+  if (!h->platforms_read) CUDA_TRY(cudaEventCreateWithFlags(&h->platforms_read, cudaEventDisableTiming));
+  if (n_platforms > h->d_platforms_cap) {
+    CUDA_TRY(cudaEventSynchronize(h->platforms_read));      // the previous launch has read the old list
+    CUDA_TRY(cudaFree(h->d_platforms));
+    h->d_platforms = nullptr;
+    h->d_platforms_cap = 0;
+    CUDA_TRY(cudaMalloc(&h->d_platforms, (size_t)n_platforms * sizeof(dqlb200_platform)));
+    h->d_platforms_cap = n_platforms;
+  }
+  CUDA_TRY(cudaStreamWaitEvent(s, h->platforms_read, 0));      // a launch on another stream may still read the list
+  // from pageable memory the copy is staged before cudaMemcpyAsync returns, so neither platforms_host nor platforms_stage is read later
+  CUDA_TRY(cudaMemcpyAsync(h->d_platforms, h->platforms_stage.data(), (size_t)n_platforms * sizeof(dqlb200_platform), cudaMemcpyHostToDevice, s));
+  const int rc = launch_eval_agents(h, working_step, first_episode, episodes_per_agent, h->d_platforms, n_platforms, stats_out, nullptr, s);
+  if (rc) return rc;
+  CUDA_TRY(cudaEventRecord(h->platforms_read, s));
   return DQLB200_OK;
 }
 

@@ -124,23 +124,30 @@ __device__ __forceinline__ uint8_t greedy_action_f32(const float* __restrict__ q
   return (uint8_t)a;
 }
 
-// Every agent's greedy policy in one launch: blocks_per_agent blocks of 256 episodes per agent on a flat 1-D grid (agent =
-// blockIdx.x / blocks_per_agent).  Agent g reads replica g * replicas: its tables (the LUT is built per block in shared memory),
-// Philox key, platform and -- for w < 0 -- its live working step.  Episode i of agent g is episode first_episode + i of
-// eval_kernel for population g * replicas under the same LUT.  Reads the tables and trainer state, writes only stats / policy_out.
+// Every agent's greedy policy in one launch, under its own platform or under each of a list of platform motions:
+// blocks_per_agent blocks of 256 episodes per (agent, platform) cell on a flat 1-D grid (cell = blockIdx.x / blocks_per_agent =
+// agent * n_platforms + c).  Agent g reads replica g * replicas: its tables (the LUT is built per block in shared memory),
+// Philox key, population_id, signed g / axis and -- for w < 0 -- its live working step.  platforms == nullptr (n_platforms = 1):
+// the agent's own platform; otherwise cell (g, c) replaces only dphase, r, rw, rw2 with platforms[c].  Episode i of cell (g, c)
+// is episode first_episode + i of eval_kernel for population g * replicas under the same LUT and that platform.  The reset
+// draw does not depend on the platform (dyn_reset: x offset and start phase in turns come from the Philox word alone), so
+// episode i starts from the same offset and phase in every column: columns differ by platform motion only.  Reads the
+// tables and trainer state, writes only stats [n_agents][n_platforms] / policy_out (from the first block of platform 0).
 template <bool GENERIC>
 __global__ void __launch_bounds__(256) eval_agents_kernel(const __grid_constant__ KC kc, const dqlb200_population_params* pop_params,
                                                           const uint32_t* __restrict__ tables, const dqlb200_population_state* __restrict__ pop_state,
                                                           int replicas, int blocks_per_agent, long long first_episode,
-                                                          long long episodes_per_agent, int w, dqlb200_eval_stats* stats,
-                                                          uint8_t* __restrict__ policy_out) {
+                                                          long long episodes_per_agent, int w, const dqlb200_platform* __restrict__ platforms,
+                                                          int n_platforms, dqlb200_eval_stats* stats, uint8_t* __restrict__ policy_out) {
   const auto& kk = ConstsOf<GENERIC>::get(kc);
   constexpr int N_STATES = DQLB200_MAX_CURRICULUM * DQLB200_STATES_PER_LEVEL;
   __shared__ uint8_t s_policy[N_STATES];
   __shared__ dqlb200_cuts cuts;
   __shared__ unsigned int s_hist[9], s_steps, s_eps;
-  const int agent = (int)(blockIdx.x / (unsigned)blocks_per_agent);
-  const int block_in_agent = (int)(blockIdx.x - (unsigned)agent * (unsigned)blocks_per_agent);
+  __shared__ dqlb200_population_params s_pp;      // the block's parameters: read in place (a register copy of both sources spills)
+  const int cell = (int)(blockIdx.x / (unsigned)blocks_per_agent);
+  const int block_in_agent = (int)(blockIdx.x - (unsigned)cell * (unsigned)blocks_per_agent);
+  const int agent = cell / n_platforms, platform = cell - agent * n_platforms;
   const int pop = agent * replicas;
   const float* qa = reinterpret_cast<const float*>(tables + (size_t)pop * 3 * DQLB200_MAX_CELLS);
   const float* qb = qa + DQLB200_MAX_CELLS;
@@ -150,12 +157,18 @@ __global__ void __launch_bounds__(256) eval_agents_kernel(const __grid_constant_
     const int wl = w >= 0 ? w : min(max(pop_state[pop].working_step, 0), kc.curriculum_steps - 1);      // clamped: never index past cuts[]
     cuts = kc.cuts[wl];
     s_steps = s_eps = 0u;
+    dqlb200_population_params pp = pop_params[pop];
+    if (platforms) {
+      const dqlb200_platform pl = platforms[platform];
+      pp.dphase = pl.dphase; pp.r = pl.r; pp.rw = pl.rw; pp.rw2 = pl.rw2;
+    }
+    s_pp = pp;
   }
   if (threadIdx.x < 9) s_hist[threadIdx.x] = 0u;
   __syncthreads();
-  if (policy_out && block_in_agent == 0)
+  if (policy_out && block_in_agent == 0 && platform == 0)
     for (int s = threadIdx.x; s < N_STATES; s += blockDim.x) policy_out[(size_t)agent * N_STATES + s] = s_policy[s];
-  const dqlb200_population_params pp = pop_params[pop];
+  const dqlb200_population_params& pp = s_pp;
   const long long i = (long long)block_in_agent * blockDim.x + threadIdx.x;
   if (i < episodes_per_agent) {
     int step;
@@ -166,7 +179,7 @@ __global__ void __launch_bounds__(256) eval_agents_kernel(const __grid_constant_
     atomicAdd(&s_eps, 1u);
   }
   __syncthreads();
-  dqlb200_eval_stats* st = stats + agent;
+  dqlb200_eval_stats* st = stats + cell;
   if (threadIdx.x < 9 && s_hist[threadIdx.x]) atomicAdd((unsigned long long*)&st->termination_hist[threadIdx.x], (unsigned long long)s_hist[threadIdx.x]);
   if (threadIdx.x == 0) {
     atomicAdd((unsigned long long*)&st->steps, (unsigned long long)s_steps);

@@ -328,6 +328,34 @@ class Engine:
             res["policy"] = host[stats_bytes:].reshape(A, n_states).copy()
         return res
 
+    def eval_platforms(self, episodes_per_agent: int, platforms: Sequence[Sequence[float]], *, working_step: Optional[int] = None,
+                       first_episode: int = 0) -> dict:
+        """eval_agents under each of a list of platform motions (dqlb200_eval_agents_platforms): every agent x every platform x
+        episodes_per_agent greedy SimulationMdp episodes from the live float32 tables, one launch, one copy back, one
+        synchronisation.  platforms: (r_mp, v_mp) pairs, converted as the Engine converts its own (platform_constants).  Cell
+        (g, c) is eval_greedy(<g's float32 LUT>, episodes_per_agent, population=g * R, first_episode=..., working_step=...) on an
+        Engine whose population g * R flies platform c; episode i starts from the same offset and platform phase under every
+        platform.  working_step None = each agent's live working step.  Returns NumPy arrays: platforms [C, 2], episodes [A, C],
+        steps [A, C], termination_hist [A, C, 9], success_rate [A, C] (goal or contact, as eval_agents)."""
+        pl = K.platform_motions(platforms)
+        n = len(pl)
+        host = (K.Platform * n)()
+        for c, (r, v) in enumerate(pl):
+            host[c] = K.Platform(*K.platform_constants(r, v, self.mp.f_ag, self.dp.n_sub))
+            if not all(np.isfinite([host[c].r, host[c].rw, host[c].rw2])) or not host[c].r > 0:
+                raise ValueError(f"platform {c} (r_mp={r}, v_mp={v}) does not fit float32")
+        A = self.P // self.R
+        stats_bytes = A * n * C.sizeof(K.EvalStats)
+        buf = torch.zeros(stats_bytes, dtype=torch.uint8, device=self.device)
+        w = -1 if working_step is None else int(working_step)
+        _ffi.check(self.lib.dqlb200_eval_agents_platforms(self.handle, w, int(first_episode), int(episodes_per_agent), host, n,
+                                                          buf.data_ptr(), self._stream()))
+        st = buf.cpu().numpy().view(np.uint64).reshape(A, n, 11).astype(np.int64)      # the copy synchronises the stream
+        res = dict(platforms=pl, episodes=st[:, :, 0], steps=st[:, :, 1], termination_hist=st[:, :, 2:])
+        hist = res["termination_hist"]
+        res["success_rate"] = (hist[:, :, 2] + hist[:, :, 3]) / np.maximum(res["episodes"], 1)
+        return res
+
     def eval_greedy_2d(self, policy_x: np.ndarray, policy_y: np.ndarray, n_episodes: int, *, two_axis: Optional[K.TwoAxisParameters] = None,
                        seed: int = 42, stream_id: int = 0, first_episode: int = 0, working_step: int = 4, trace_steps: int = 0):
         """Greedy two-axis SimulationMdp episodes: agent_x and agent_y both predict every step (scripts/simulation.py:48-63).

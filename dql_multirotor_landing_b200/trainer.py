@@ -48,6 +48,7 @@ class Trainer:
     _eval_every: Optional[int] = None       # greedy evaluation of every agent after each `eval_every`-th chunk (None: off)
     _eval_episodes: int = 1024
     _eval_two_axis: Optional[K.TwoAxisParameters] = None      # also the two-axis landing (x policy on x, its mirror on y)
+    _eval_platforms: Optional[list] = None      # also the landing under each of these (r_mp, v_mp) platform motions
 
     def __init__(
         self,
@@ -86,6 +87,7 @@ class Trainer:
         eval_every: Optional[int] = None,
         eval_episodes: int = 1024,
         eval_two_axis: Optional[K.TwoAxisParameters] = None,
+        eval_platforms: Optional[Sequence[Sequence[float]]] = None,
     ) -> None:
         np.random.seed(seed)                                        # PKG/trainer.py:45
         if not double_q_learning_agent:
@@ -138,6 +140,10 @@ class Trainer:
             if self._dynamics.accel_mode != "exact" or self._dynamics.dynamics_model != "first_order":
                 raise ValueError("eval_two_axis runs the first-order model with the exact acceleration only")
             self._eval_two_axis = eval_two_axis
+        if eval_platforms is not None:      # likewise stored only when set
+            if eval_every is None:
+                raise ValueError("eval_platforms needs eval_every")
+            self._eval_platforms = [(float(r), float(v)) for r, v in K.platform_motions(eval_platforms)]
         self._engine = None
         self.history = []             # one dict per chunk (population 0)
 
@@ -277,6 +283,10 @@ class Trainer:
                                             two_axis=self._eval_two_axis)["success_rate"]
                     info["Greedy two-axis success rate"] = float(rates2[0])
                     entry["Greedy two-axis success rates"] = [float(r) for r in rates2]
+                if self._eval_platforms is not None:     # every agent under each listed platform motion, one launch
+                    by_platform = eng.eval_platforms(self._eval_episodes, self._eval_platforms)["success_rate"]
+                    info["Greedy success rate by platform"] = [float(r) for r in by_platform[0]]
+                    entry["Greedy success rates by platform"] = [[float(r) for r in row] for row in by_platform]
             self.history.append(dict(info, working_step=self._working_curriculum_step, **entry))
             if len(self.history) > 2048:          # bounded: the history is pickled with every checkpoint
                 del self.history[:1024]
@@ -312,6 +322,9 @@ class Trainer:
                 writer.add_scalar("Episode/Greedy Success Rate", info["Greedy success rate"], step)
             if "Greedy two-axis success rate" in info:
                 writer.add_scalar("Episode/Greedy Two-Axis Success Rate", info["Greedy two-axis success rate"], step)
+            if "Greedy success rate by platform" in info:
+                for (r, v), rate in zip(self._eval_platforms, info["Greedy success rate by platform"]):
+                    writer.add_scalar(f"Episode/Greedy Success Rate (r={r:g}, v={v:g})", rate, step)
             writer.add_text("Episode/Termination Condition", info["Termination condition"], step)
             writer.close()
         if clean:

@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define DQLB200_ABI_VERSION 10
+#define DQLB200_ABI_VERSION 11
 #define DQLB200_MAX_CURRICULUM 5
 #define DQLB200_STATES_PER_LEVEL 189          /* 3*3*3*7      (PKG/double_q_learning.py:38-40) */
 #define DQLB200_CELLS_PER_LEVEL 567           /* 189 * 3 actions */
@@ -207,6 +207,13 @@ typedef struct dqlb200_eval_stats {
   uint64_t termination_hist[9];
 } dqlb200_eval_stats;
 
+/* One platform motion x = r sin(w t) of dqlb200_eval_agents_platforms (16 B): the fields of dqlb200_population_params with the
+ * same names and meaning, computed on the host the same way (constants.platform_constants(r_mp, v_mp, f_ag, n_sub)). */
+typedef struct dqlb200_platform {
+  uint32_t dphase;                  /* platform phase advance per sub-step, uint32 turns */
+  float r, rw, rw2;                 /* platform amplitude, r*w, r*w^2 */
+} dqlb200_platform;
+
 /* Two-axis greedy evaluation (SURVEY.md 8f-2): pitch drives x, roll drives y, one platform under both.
  * trajectory 0: x = r_x sin(w_x t), y = 0                     (PKG/moving_platform.py:113-125 with omega_y = 0)
  *            1: x = r_x sin(w_x t), y = r_y sin(w_y t)        (the "future extension" kept in :113-125)
@@ -238,6 +245,7 @@ int dqlb200_abi_version(void);
 size_t dqlb200_config_bytes(void);
 size_t dqlb200_population_state_bytes(void);
 size_t dqlb200_eval2d_params_bytes(void);
+size_t dqlb200_platform_bytes(void);
 /* Bytes of the env-state buffer for a layout: n_populations * ceil(envs_per_population / 32) * DQLB200_ENV_TILE_BYTES. */
 size_t dqlb200_env_state_bytes(int n_populations, int envs_per_population);
 const char* dqlb200_last_error(void);
@@ -341,6 +349,27 @@ int dqlb200_eval_greedy(dqlb200_handle* h, int population, const uint8_t* policy
  * option without its bound buffer (DQLB200_ERR_STATE).  episodes_per_agent <= 0 does nothing. */
 int dqlb200_eval_agents(dqlb200_handle* h, int working_step, int64_t first_episode, int64_t episodes_per_agent,
                         void* stats_out, uint8_t* policy_out, void* stream);
+
+/* dqlb200_eval_agents under each of a LIST of platform motions, in one launch: agents x platforms x episodes from the live
+ * float32 tables, for how an agent lands at platform speeds and amplitudes it was not trained on.
+ *   platforms_host : host dqlb200_platform[n_platforms].  Copied into a library-owned host buffer and from there to a
+ *                    library-owned device buffer on `stream`: the list (pageable or pinned) is never read after the call
+ *                    returns, so the caller may rewrite it at once.
+ *   cell (g, c)    : agent g (as in dqlb200_eval_agents: replica g*R, its tables, Philox key, population_id, signed g / axis and
+ *                    live or given working step) flying platform c: only dphase, r, rw, rw2 of its dqlb200_population_params
+ *                    are replaced.  Row (g, c) is, episode for episode, dqlb200_eval_greedy(population = g*R, <g's float32
+ *                    first-max LUT>, first_episode, episodes_per_agent, working_step) on a handle whose population g*R has
+ *                    platform c.  The reset draw does not depend on the platform, so episode i starts from the same x offset
+ *                    and platform phase (in turns) under every platform: differences between columns are differences of
+ *                    platform motion alone.  With accel_mode / dynamics_model every episode starts a fresh simulator.
+ *   stats_out      : device dqlb200_eval_stats[n_agents][n_platforms], agent-major, accumulated (the caller zeroes).
+ * Nothing bound is written.  dqlb200_eval_agents is this call with each agent's own platform.
+ * Refused (DQLB200_ERR_ARG): a NULL handle, platforms_host or stats_out; n_platforms < 1; a platform whose r is not finite or
+ * <= 0, or whose rw / rw2 is not finite or < 0; working_step outside -1 .. curriculum_steps - 1; more than 0x7FFFFFFF blocks
+ * (ceil(episodes_per_agent / 256) * n_agents * n_platforms).  Tables or trainer state not bound, an option without its bound
+ * buffer: DQLB200_ERR_STATE.  episodes_per_agent <= 0 does nothing. */
+int dqlb200_eval_agents_platforms(dqlb200_handle* h, int working_step, int64_t first_episode, int64_t episodes_per_agent,
+                                  const dqlb200_platform* platforms_host, int n_platforms, void* stats_out, void* stream);
 
 /* Un-fused environment entry points: the gym surface of the reference with caller-supplied actions, no agent, no table.
  *   dqlb200_env_reset  replaces TrainingLandingEnv.reset / SimulationLandingEnv.reset (PKG/landing_simulation_env.py:167-243,

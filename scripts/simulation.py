@@ -4,6 +4,7 @@ agents, runs greedy episodes.  Default: ten episodes through the gym surface exa
 
     python scripts/simulation.py
     python scripts/simulation.py --episodes 1048576 --two-axis
+    python scripts/simulation.py --episodes 4096 --platforms 2:0.4 2:0.8 2:1.2 2:1.6     # landing rate per platform (r_mp:v_mp)
 """
 import argparse
 import pathlib
@@ -15,6 +16,15 @@ from dql_multirotor_landing_b200 import constants as K                          
 from dql_multirotor_landing_b200.double_q_learning import DoubleQLearningAgent          # noqa: E402
 from dql_multirotor_landing_b200.engine import Engine, greedy_policy, mirrored_policy   # noqa: E402
 from dql_multirotor_landing_b200.landing_simulation_env import make                     # noqa: E402
+
+
+def platform_arg(text):
+    """R:V -> (r_mp, v_mp)"""
+    try:
+        r, v = text.split(":")
+        return float(r), float(v)
+    except ValueError:
+        raise argparse.ArgumentTypeError(f"expected R:V (platform amplitude r_mp and speed v_mp), got {text!r}") from None
 
 
 def log(info, clean=False):
@@ -39,10 +49,21 @@ if __name__ == "__main__":
     ap.add_argument("--two-axis", action="store_true", help="both agents act (the reference leaves the y action disabled)")
     ap.add_argument("--assets", default=None, help="directory with Q_table_a.npy / Q_table_b.npy / state_action_count.npy")
     ap.add_argument("--seed", type=int, default=42)
+    ap.add_argument("--platforms", type=platform_arg, nargs="+", default=None, metavar="R:V",
+                    help="greedy landing rate of the agent under each platform motion (amplitude r_mp, speed v_mp), one launch")
     a = ap.parse_args()
     agent_x = DoubleQLearningAgent.load(a.assets) if a.assets else DoubleQLearningAgent.load()
     agent_y = DoubleQLearningAgent.load(a.assets) if a.assets else DoubleQLearningAgent.load()
-    if a.episodes <= 10 and not a.two_axis:
+    if a.platforms:
+        K.platform_motions(a.platforms)          # ValueError for a malformed list, before the device is touched
+        eng = Engine(1, 1, seeds=[a.seed])
+        eng.set_tables(0, agent_x.Q_table_a, agent_x.Q_table_b, agent_x.state_action_counter)
+        res = eng.eval_platforms(a.episodes, a.platforms, working_step=eng.tp.curriculum_steps - 1)
+        print(f"episodes per platform: {a.episodes}  (float32 greedy policy of the agent's tables, working step {eng.tp.curriculum_steps - 1})")
+        for (r, v), rate, steps in zip(res["platforms"], res["success_rate"][0], res["steps"][0]):
+            print(f"  r_mp = {r:g}  v_mp = {v:g}: landed {rate:.4f}  env-steps {steps}")
+        eng.close()
+    elif a.episodes <= 10 and not a.two_axis:
         env = make("Landing-Simulation-v0", seed=a.seed)
         for current_episode in range(a.episodes):
             current_state_x, current_state_y = env.reset()

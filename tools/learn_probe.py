@@ -5,6 +5,9 @@ Engine.eval_agents).  One script for the cases DESIGN.md section 3 quotes:
     python tools/learn_probe.py single               one env / 64 / 1,024 envs per CTA (S1 semantics), 8 seeds each
     python tools/learn_probe.py merge                one agent as R replicas x 128 envs, merge interval 1 / 8 / 64
     python tools/learn_probe.py speed                success-rate plateau vs platform speed (128 replicas, merge every step)
+    python tools/learn_probe.py generalisation       one agent trained per speed of {0.4, 0.8, 1.2, 1.6} (r_mp = 2, 128 replicas
+                                                     each, one Engine), then the greedy landing rate of every agent at every
+                                                     speed: the 4 x 4 matrix (trained at x evaluated at) of one eval_platforms call
     python tools/learn_probe.py R,n_r,merge_every,total_steps[,v_mp]     any replica-merge shape (R = 0: P = 8 independent CTAs of n_r envs)
 """
 import json
@@ -48,6 +51,22 @@ def run(R, n_r, merge_every, total_steps, v_mp=1.6, chunks=6, n_sub=1):
     eng.close()
 
 
+def generalisation(speeds=(0.4, 0.8, 1.2, 1.6), r_mp=2.0, R=128, n_r=128, total_steps=250000, episodes=1024):
+    tp = K.TrainerParameters(success_rate=2.0, max_num_episodes=10 ** 15)
+    A = len(speeds)
+    eng = Engine(A * R, n_r, threads_per_block=128, seeds=[42 + g for g in range(A) for _ in range(R)], population_ids=list(range(A * R)),
+                 replicas_per_population=R, r_mp=[r_mp] * (A * R), v_mp=[v for v in speeds for _ in range(R)], tp=tp)
+    eng.reset(0)
+    eng.train_merged(total_steps, 1)
+    res = eng.eval_platforms(episodes, [(r_mp, v) for v in speeds])      # at the live working step (promotion off: 0)
+    own = eng.eval_agents(episodes)["success_rate"]
+    assert np.array_equal(np.diag(res["success_rate"]), own)        # the diagonal is each agent under its own platform
+    print(json.dumps(dict(r_mp=r_mp, speeds=list(speeds), replicas=R, envs_per_cta=n_r, total_steps=total_steps, episodes=episodes,
+                          rows_trained_at_cols_evaluated_at=[[round(float(x), 4) for x in row] for row in res["success_rate"]])),
+          flush=True)
+    eng.close()
+
+
 if __name__ == "__main__":
     for a in sys.argv[1:] or ["single"]:
         if a == "single":
@@ -55,6 +74,8 @@ if __name__ == "__main__":
         elif a == "merge":
             for R, m in ((8, 8), (64, 8), (512, 8), (512, 1), (512, 64)):
                 run(R, 128, m, 300000)
+        elif a == "generalisation":
+            generalisation()
         elif a == "speed":
             for v in (0.0, 0.4, 0.8, 1.0, 1.2, 1.6):
                 run(128, 128, 1, 250000, v_mp=v, chunks=5)
